@@ -1,6 +1,6 @@
 """bench.py — denoise steps/sec of the B200-native UniGenFlux forward (BASELINE.json metric) on synthetic inputs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload cfg3|cfg2|tiny]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload cfg3|cfg2|tiny] [--dump-outputs DIR]
   N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one `UniGenFlux.forward` (one denoise step) of every rank's micro-batch; ranks hold independent samples
@@ -110,6 +110,27 @@ def summarize_clocks(lines):
     if not sm:
         return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
     return {"sm_mhz": statistics.median(sm), "sm_max_mhz": max(mx), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BUDGET = 60 << 20  # bytes of array data per dump: with the .npy headers the directory stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays, budget: int = DUMP_BUDGET):
+    """`--dump-outputs DIR`: every output tensor as DIR/<name>.npy, floating point as float32 and integers as float64 (exact),
+    so that two builds can be compared output for output. When the arrays together exceed `budget` bytes, each keeps its
+    share of the budget as a fixed, seeded sample of its flattened elements (same positions in every run)."""
+    import numpy as np
+    import torch
+    arrays = {k: v.detach().cpu() for k, v in arrays.items()}
+    arrays = {k: v.to(torch.float32 if v.is_floating_point() else torch.float64) for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        if total > budget:
+            keep = v.numel() * budget // total
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            v = v.flatten()[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), v.numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -257,9 +278,12 @@ def run_native(args):
     d2h_bytes = out_host.numel() * out_host.element_size()
     to_dev = lambda v, **k: [t.to(dev, **k) for t in v] if isinstance(v, list) else v.to(dev, **k)  # noqa: E731
     resident = {k: to_dev(v) for k, v in host.items()}
+    last = None  # (velocity, add_losses, add_outputs) of the latest resident step: forward hands out copies
 
     def step_resident():
-        return model(**resident)[0]
+        nonlocal last
+        last = model(**resident)
+        return last[0]
 
     def step_e2e():
         devin = {k: to_dev(v, non_blocking=True) for k, v in host.items()}
@@ -295,6 +319,9 @@ def run_native(args):
     ops.reset_launch_count()
     ms_total = timed(step_resident, args.steps)
     launches = ops.launch_count()
+    if args.dump_outputs and rank == 0:
+        velocity, add_losses, add_outputs = last
+        dump_outputs(args.dump_outputs, {"velocity": velocity, **add_losses, **add_outputs})
     for _ in range(2):
         step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
@@ -724,7 +751,13 @@ def main():
     ap.add_argument("--no-sp-pvariant", action="store_true", help="N > 1: skip the cfg4 P-variant sequence-parallel leg")
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the same-box torch-eager bf16 comparator")
     ap.add_argument("--loop", type=int, default=0, help="also time the whole-loop CUDA graph: LOOP denoise steps per graph launch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (velocity, moe_loss, expert_counts) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("cfg4p", "cfg5")):
+        ap.error("--dump-outputs is available for the native Flux workloads (cfg2, cfg3, cfg4, tiny)")
     if args.workload in ("cfg4p", "cfg5"):
         if args.impl == "reference":
             if int(os.environ.get("RANK", "0")) == 0:
