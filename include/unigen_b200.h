@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define UG_ABI_VERSION 9
+#define UG_ABI_VERSION 10
 
 typedef enum {
   UG_OK = 0,
@@ -134,6 +134,29 @@ typedef struct ug_gemm_args {
 
 int ug_gemm_bf16(const ug_gemm_args* args, void* stream);
 
+/* Row-wise FP8 (e4m3) GEMM: the same tiles, tile walk and epilogues as ug_gemm_bf16 with `a` / `w` read as float8_e4m3fn
+ * (strides count elements = bytes; a / w row strides and k multiples of 16) and kind::f8f6f4 MMAs accumulating in fp32. The
+ * accumulator is dequantised first, then the epilogue of ug_gemm_bf16 runs:
+ *   acc[b, r, c] * a_scale[b, r] * w_scale[c]  ->  bias -> GELU-tanh -> gate * alpha -> residual   (or fused QK-norm + RoPE)
+ * C, bias, residual and the QK-norm operands stay bf16 / fp32 as in ug_gemm_bf16. lora_t, colmask_block, a2 / w2 are rejected.
+ * One fp32 scale per token row of A (dynamic, from ug_quant_rows_fp8 / ug_ln_modulate_fp8) and one per output channel of W
+ * (`quantize_fp8()`): the "row-wise" scaling torch._scaled_mm offers. */
+typedef struct ug_gemm_fp8_scales {
+  const float* a_scale;          /* fp32 [batch, rows]: element (b, r) at a_scale[b * a_scale_batch_stride + r] */
+  int64_t a_scale_batch_stride;
+  const float* w_scale;          /* fp32 [n] (batched W: [batch, n] at w_scale[b * w_scale_batch_stride + c]) */
+  int64_t w_scale_batch_stride;
+} ug_gemm_fp8_scales;
+int ug_gemm_fp8(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream);
+
+/* Dynamic row-wise quantisation of bf16 [batch, rows, k] (strided) to e4m3 [batch, rows, k] plus one fp32 scale per row:
+ *   amax = max |x|;  amax == 0: scale = 1, q = 0;  else inv = 448 / amax, scale = amax / 448 (IEEE divisions),
+ *   q = cvt.rn.satfinite.e4m3(x * inv)        == torch (x.float() * inv).clamp(-448, 448).to(torch.float8_e4m3fn)
+ * scale element (b, r) at scale[b * scale_batch_stride + r]. k a multiple of 8, at most 16384; rows 16-byte aligned. */
+int ug_quant_rows_fp8(const void* x, int64_t x_row_stride, int64_t x_batch_stride, void* q, int64_t q_row_stride,
+                      int64_t q_batch_stride, float* scale, int64_t scale_batch_stride, int32_t batch, int32_t rows, int32_t k,
+                      void* stream);
+
 /* LoRA down-projection for ug_gemm_bf16's fused update: t[b, r, :] = x[b, r, :] @ A[g(r)]^T  (fp32 out).
  * a_stack: bf16 [groups, rank_total, k] (rank_total = n_sub_linears * rank for a fused projection); rows whose
  * segment has group -1 get zeros. peft 0.15 lora.Linear: lora_A (SURVEY.md §A.6). */
@@ -197,6 +220,13 @@ int ug_expand_segment_mask(int32_t seq, int32_t n_seg, const int32_t* seg_bounds
 int ug_ln_modulate(const void* x, int64_t x_row_stride, int64_t x_batch_stride, void* out, int64_t o_row_stride,
                    int64_t o_batch_stride, const float* shift, const float* scale, int64_t mod_batch_stride,
                    int32_t batch, int32_t rows, int32_t d, float eps, void* stream);
+
+/* ug_ln_modulate followed by the row quantisation of ug_quant_rows_fp8 in one pass: every value is rounded to bf16 first, so
+ * (q, q_scale) equal ug_quant_rows_fp8(ug_ln_modulate(x)) bit for bit. The operand of the fp8 GEMMs that read a modulated
+ * LayerNorm (q|k|v, ff.net.0, proj_mlp). q: e4m3 [batch, rows, d]; q_scale: fp32, (b, r) at q_scale[b * q_scale_batch_stride + r]. */
+int ug_ln_modulate_fp8(const void* x, int64_t x_row_stride, int64_t x_batch_stride, void* q, int64_t q_row_stride,
+                       int64_t q_batch_stride, float* q_scale, int64_t q_scale_batch_stride, const float* shift, const float* scale,
+                       int64_t mod_batch_stride, int32_t batch, int32_t rows, int32_t d, float eps, void* stream);
 
 /* ug_ln_modulate with one modulation vector per ROW SEGMENT: rows [seg_bounds[i], seg_bounds[i+1]) of every sample use
  * shift/scale + i * mod_seg_stride (+ b * mod_batch_stride) — the text / image / condition streams of a P-variant block

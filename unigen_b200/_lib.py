@@ -12,7 +12,7 @@ UG_ACT_NONE = 0
 UG_ACT_GELU_TANH = 1
 UG_MAX_SEGMENTS = 8
 UG_GROUPNORM_MAX_CHUNKS = 1024
-UG_ABI_VERSION = 9  # include/unigen_b200.h; checked against ug_abi_version() of the loaded library
+UG_ABI_VERSION = 10  # include/unigen_b200.h; checked against ug_abi_version() of the loaded library
 
 
 class UgError(RuntimeError):
@@ -38,6 +38,11 @@ class GemmArgs(C.Structure):
         ("a2", C.c_void_p), ("a2_row_stride", C.c_int64), ("a2_batch_stride", C.c_int64),
         ("w2", C.c_void_p), ("w2_row_stride", C.c_int64), ("k2", C.c_int32), ("colmask_block", C.c_int32),
     ]
+
+
+class GemmFp8Scales(C.Structure):
+    _fields_ = [("a_scale", C.c_void_p), ("a_scale_batch_stride", C.c_int64),
+                ("w_scale", C.c_void_p), ("w_scale_batch_stride", C.c_int64)]
 
 
 class Conv2dArgs(C.Structure):
@@ -117,6 +122,9 @@ SIGNATURES = {
     "ug_launch_count": (C.c_int64, []),
     "ug_reset_launch_count": (None, []),
     "ug_gemm_bf16": (C.c_int, [C.POINTER(GemmArgs), _VP]),
+    "ug_gemm_fp8": (C.c_int, [C.POINTER(GemmArgs), C.POINTER(GemmFp8Scales), _VP]),
+    "ug_quant_rows_fp8": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _I64, _I32, _I32, _I32, _VP]),
+    "ug_ln_modulate_fp8": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _I64, _VP, _VP, _I64, _I32, _I32, _I32, _F32, _VP]),
     "ug_lora_down": (C.c_int, [_VP, _I64, _I64, _VP, _VP, _I64, _I64, _I32, _I32, _I32, _I32, _I32,
                                C.POINTER(C.c_int32), C.POINTER(C.c_int32), _VP]),
     "ug_lora_down_wide": (C.c_int, [_VP, _I64, _I64, _VP, _VP, _I64, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32,

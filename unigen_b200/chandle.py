@@ -20,6 +20,8 @@ class FluxStepHandle:
         a = model.arch
         if getattr(model, "use_consis_module", False) and model.use_shared_expert:
             raise ops.UgError("ug_flux handle: use_consis_module is sequenced by the Python host only (unigen_b200.model)")
+        if getattr(model, "linear_dtype", torch.bfloat16) != torch.bfloat16:
+            raise ops.UgError("ug_flux handle: fp8-quantised block linears (quantize_fp8) run on the Python host only (unigen_b200.model)")
         d = FluxDesc()
         d.num_layers, d.num_single_layers, d.heads, d.head_dim = a.num_layers, a.num_single_layers, a.num_attention_heads, a.attention_head_dim
         d.in_channels, d.joint_dim, d.pooled_dim, d.guidance_embeds = a.in_channels, a.joint_attention_dim, a.pooled_projection_dim, int(a.guidance_embeds)

@@ -4,6 +4,8 @@
 #include <cstdlib>
 #include <cstring>
 
+#include <cuda_fp8.h>
+
 #include <algorithm>
 
 #include "ug_host.h"
@@ -28,6 +30,84 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Row-wise e4m3 quantisation (the activation side of the fp8 GEMM): amax = max |x| of the row; amax == 0 -> scale 1, q = 0;
+// else inv = 448 / amax, scale = amax / 448 (IEEE round-to-nearest divisions) and q = cvt.rn.satfinite.e4m3(x * inv).
+// ---------------------------------------------------------------------------------------------------
+struct Fp8Out {  // e4m3 rows + one fp32 scale per row; q == nullptr: plain bf16 output
+  uint8_t* q;
+  long long q_rs, q_bs;
+  float* scale;
+  long long s_bs;
+};
+
+__device__ __forceinline__ float warp_max(float v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+__device__ __forceinline__ float fp8_inv_scale(float amax) { return amax == 0.f ? 0.f : __fdiv_rn(448.0f, amax); }
+__device__ __forceinline__ float fp8_row_scale(float amax) { return amax == 0.f ? 1.f : __fdiv_rn(amax, 448.0f); }
+// the values a bf16 store of f would hold (the fused LN kernels quantise exactly what ug_ln_modulate writes)
+__device__ __forceinline__ void round_bf16x8(float (&f)[8]) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) f[j] = __bfloat162float(__float2bfloat16_rn(f[j]));
+}
+__device__ __forceinline__ float absmax8(const float (&f)[8], float m) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) m = fmaxf(m, fabsf(f[j]));
+  return m;
+}
+// 8 values -> 8 e4m3 bytes (x * inv, saturating round-to-nearest); inv == 0 (all-zero row) stores +0 everywhere
+__device__ __forceinline__ uint2 e4m3x8(const float (&f)[8], float inv) {
+  if (inv == 0.f) return make_uint2(0u, 0u);
+  uint32_t h[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    h[j] = (uint32_t)__nv_cvt_float2_to_fp8x2(make_float2(f[2 * j] * inv, f[2 * j + 1] * inv), __NV_SATFINITE, __NV_E4M3);
+  return make_uint2(h[0] | (h[1] << 16), h[2] | (h[3] << 16));
+}
+
+// one block per row, the row resident in registers (k <= 8 * kThreads * kMaxV)
+template <int kThreads, int kMaxV>
+__global__ void __launch_bounds__(kThreads) quant_rows_fp8_kernel(const __nv_bfloat16* __restrict__ x, long long x_rs, long long x_bs,
+                                                                  Fp8Out o, int k) {
+  constexpr int kWarps = kThreads / 32;
+  __shared__ float red[kWarps];
+  const int t = threadIdx.x, r = blockIdx.x, b = blockIdx.y;
+  const uint4* xp = reinterpret_cast<const uint4*>(x + (long long)b * x_bs + (long long)r * x_rs);
+  const int nvec = k >> 3;
+  uint4 buf[kMaxV];
+  float amax = 0.f;
+#pragma unroll
+  for (int i = 0; i < kMaxV; ++i) {
+    const int v = t + kThreads * i;
+    if (v < nvec) {
+      buf[i] = xp[v];
+      float f[8];
+      unpack8(buf[i], f);
+      amax = absmax8(f, amax);
+    }
+  }
+  amax = warp_max(amax);
+  if ((t & 31) == 0) red[t >> 5] = amax;
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < kWarps; ++w) amax = fmaxf(amax, red[w]);
+  const float inv = fp8_inv_scale(amax);
+  uint2* qp = reinterpret_cast<uint2*>(o.q + (long long)b * o.q_bs + (long long)r * o.q_rs);
+#pragma unroll
+  for (int i = 0; i < kMaxV; ++i) {
+    const int v = t + kThreads * i;
+    if (v < nvec) {
+      float f[8];
+      unpack8(buf[i], f);
+      qp[v] = e4m3x8(f, inv);
+    }
+  }
+  if (t == 0) o.scale[(long long)b * o.s_bs + r] = fp8_row_scale(amax);
+}
+
+// ---------------------------------------------------------------------------------------------------
 // LayerNorm (no affine) + (1 + scale) * x + shift.  One warp per row, row kept in registers (d <= 8*32*kMaxV).
 // Algorithmic HBM bytes per row: 2*d (read) + 2*d (write).
 // ---------------------------------------------------------------------------------------------------
@@ -36,7 +116,9 @@ struct RowSegs {
   int bounds[UG_MAX_SEGMENTS + 1];
 };
 
-template <int kMaxV>
+// kFp8 (every kernel below): the row is written as e4m3 + one fp32 scale (Fp8Out) instead of bf16 — the same values, rounded to
+// bf16 first, then quantised like quant_rows_fp8_kernel (a first pass over the row finds the amax, a second one stores).
+template <int kMaxV, bool kFp8 = false>
 __global__ void __launch_bounds__(256) ln_modulate_kernel(const __nv_bfloat16* __restrict__ x, long long x_rs,
                                                           long long x_bs, __nv_bfloat16* __restrict__ out,
                                                           long long o_rs, long long o_bs,
@@ -46,7 +128,7 @@ __global__ void __launch_bounds__(256) ln_modulate_kernel(const __nv_bfloat16* _
                                                           const int* __restrict__ slot_token = nullptr, int capacity = 1,
                                                           int tokens_per_batch = 1, int empty_index = 0,
                                                           long long mod_es = 0, RowSegs segs = RowSegs{0, {0}},
-                                                          long long mod_seg_stride = 0) {
+                                                          long long mod_seg_stride = 0, Fp8Out fo = Fp8Out{}) {
   const int warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (warp_global >= batch * rows) return;
@@ -92,30 +174,46 @@ __global__ void __launch_bounds__(256) ln_modulate_kernel(const __nv_bfloat16* _
   }
   const float rstd = rsqrtf(warp_sum(var) / (float)d + eps);
   uint4* op = reinterpret_cast<uint4*>(out + (long long)b * o_bs + (long long)r * o_rs);
+  uint2* qp = kFp8 ? reinterpret_cast<uint2*>(fo.q + (long long)b * fo.q_bs + (long long)r * fo.q_rs) : nullptr;
   const float* sh = shift + mod_off;
   const float* sc = scale + mod_off;
+  float amax = 0.f, inv = 0.f;
+#pragma unroll 1
+  for (int pass = kFp8 ? 0 : 1; pass < 2; ++pass) {
+    if (kFp8 && pass == 1) {
+      amax = warp_max(amax);
+      inv = fp8_inv_scale(amax);
+    }
 #pragma unroll
-  for (int i = 0; i < kMaxV; ++i) {
-    const int v = lane + 32 * i;
-    if (v < nvec) {
-      float f[8];
-      unpack8(buf[i], f);
-      const float4 s0 = *reinterpret_cast<const float4*>(sc + 8 * v), s1 = *reinterpret_cast<const float4*>(sc + 8 * v + 4);
-      const float4 h0 = *reinterpret_cast<const float4*>(sh + 8 * v), h1 = *reinterpret_cast<const float4*>(sh + 8 * v + 4);
-      const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
-      const float h[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
+    for (int i = 0; i < kMaxV; ++i) {
+      const int v = lane + 32 * i;
+      if (v < nvec) {
+        float f[8];
+        unpack8(buf[i], f);
+        const float4 s0 = *reinterpret_cast<const float4*>(sc + 8 * v), s1 = *reinterpret_cast<const float4*>(sc + 8 * v + 4);
+        const float4 h0 = *reinterpret_cast<const float4*>(sh + 8 * v), h1 = *reinterpret_cast<const float4*>(sh + 8 * v + 4);
+        const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+        const float h[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
 #pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean) * rstd * (1.f + s[j]) + h[j];
-      op[v] = pack8(f);
+        for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean) * rstd * (1.f + s[j]) + h[j];
+        if constexpr (kFp8) {
+          round_bf16x8(f);
+          if (pass == 0) amax = absmax8(f, amax);
+          else qp[v] = e4m3x8(f, inv);
+        } else {
+          op[v] = pack8(f);
+        }
+      }
     }
   }
+  if (kFp8 && lane == 0) fo.scale[(long long)b * fo.s_bs + r] = fp8_row_scale(amax);
 }
 
 // Same op, TWO warps per row (adjacent warps 2i, 2i+1 of a block; partial sums meet in shared memory). With one warp per
 // row and the row in registers a 3072-wide pass needs ~80 registers per thread -> 24 resident warps per SM -> 4608 rows take
 // 1.3 waves and the HBM pipe idles through the partial second wave; half the row per warp halves the registers, doubles the
 // resident rows' worth of loads in flight and shortens the tail.
-template <int kMaxV>
+template <int kMaxV, bool kFp8 = false>
 __global__ void __launch_bounds__(256, 4) ln_modulate2_kernel(const __nv_bfloat16* __restrict__ x, long long x_rs,
                                                            long long x_bs, __nv_bfloat16* __restrict__ out,
                                                            long long o_rs, long long o_bs,
@@ -123,7 +221,8 @@ __global__ void __launch_bounds__(256, 4) ln_modulate2_kernel(const __nv_bfloat1
                                                            const float* __restrict__ scale, long long mod_bs, int batch,
                                                            int rows, int d, float eps, const int* __restrict__ slot_token,
                                                            int capacity, int tokens_per_batch, int empty_index,
-                                                           long long mod_es, RowSegs segs, long long mod_seg_stride) {
+                                                           long long mod_es, RowSegs segs, long long mod_seg_stride,
+                                                           Fp8Out fo = Fp8Out{}) {
   __shared__ float red_sum[8], red_var[8];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long row_global = (long long)blockIdx.x * 4 + (warp >> 1);
@@ -175,25 +274,44 @@ __global__ void __launch_bounds__(256, 4) ln_modulate2_kernel(const __nv_bfloat1
   if (lane == 0) red_var[warp] = var;
   __syncthreads();
   const float rstd = rsqrtf((red_var[warp] + red_var[warp ^ 1]) / (float)d + eps);
-  if (!valid) return;
+  if (!kFp8 && !valid) return;  // (fp8: every thread reaches the amax barrier below)
   uint4* op = reinterpret_cast<uint4*>(out + (long long)b * o_bs + (long long)r * o_rs);
+  uint2* qp = kFp8 ? reinterpret_cast<uint2*>(fo.q + (long long)b * fo.q_bs + (long long)r * fo.q_rs) : nullptr;
   const float* sh = shift + mod_off;
   const float* sc = scale + mod_off;
+  float amax = 0.f, inv = 0.f;
+#pragma unroll 1
+  for (int pass = kFp8 ? 0 : 1; pass < 2; ++pass) {
+    if (kFp8 && pass == 1) {  // red_sum is free again: every thread read it before the variance barrier
+      amax = warp_max(amax);
+      if (lane == 0) red_sum[warp] = amax;
+      __syncthreads();
+      amax = fmaxf(red_sum[warp], red_sum[warp ^ 1]);
+      inv = fp8_inv_scale(amax);
+    }
 #pragma unroll
-  for (int i = 0; i < kMaxV; ++i) {
-    const int v = l64 + 64 * i;
-    if (v < nvec) {
-      float f[8];
-      unpack8(buf[i], f);
-      const float4 s0 = *reinterpret_cast<const float4*>(sc + 8 * v), s1 = *reinterpret_cast<const float4*>(sc + 8 * v + 4);
-      const float4 h0 = *reinterpret_cast<const float4*>(sh + 8 * v), h1 = *reinterpret_cast<const float4*>(sh + 8 * v + 4);
-      const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
-      const float h[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
+    for (int i = 0; i < kMaxV; ++i) {
+      const int v = l64 + 64 * i;
+      if (valid && v < nvec) {
+        float f[8];
+        unpack8(buf[i], f);
+        const float4 s0 = *reinterpret_cast<const float4*>(sc + 8 * v), s1 = *reinterpret_cast<const float4*>(sc + 8 * v + 4);
+        const float4 h0 = *reinterpret_cast<const float4*>(sh + 8 * v), h1 = *reinterpret_cast<const float4*>(sh + 8 * v + 4);
+        const float s[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+        const float h[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
 #pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean) * rstd * (1.f + s[j]) + h[j];
-      op[v] = pack8(f);
+        for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean) * rstd * (1.f + s[j]) + h[j];
+        if constexpr (kFp8) {
+          round_bf16x8(f);
+          if (pass == 0) amax = absmax8(f, amax);
+          else qp[v] = e4m3x8(f, inv);
+        } else {
+          op[v] = pack8(f);
+        }
+      }
     }
   }
+  if (kFp8 && valid && l64 == 0) fo.scale[(long long)b * fo.s_bs + r] = fp8_row_scale(amax);
 }
 
 // Same op for the plain per-sample form (no slots / row segments), kR rows per block: thread t owns the 16-byte column chunks
@@ -201,11 +319,11 @@ __global__ void __launch_bounds__(256, 4) ln_modulate2_kernel(const __nv_bfloat1
 // row of a sample — are loaded ONCE per kR rows, and they are requested together with the rows (one memory latency per block
 // instead of two: in the two-warp kernel the modulation loads only issue after both reductions, ncu: 50 % of its stall samples
 // are long-scoreboard waits on `1 + scale`). kR * kChunks + 4 * kChunks 16-byte loads in flight per thread.
-template <int kThreads, int kChunks, int kR>
+template <int kThreads, int kChunks, int kR, bool kFp8 = false>
 __global__ void __launch_bounds__(kThreads) ln_modulate_rows_kernel(const __nv_bfloat16* __restrict__ x, long long x_rs, long long x_bs,
                                                                     __nv_bfloat16* __restrict__ out, long long o_rs, long long o_bs,
                                                                     const float* __restrict__ shift, const float* __restrict__ scale,
-                                                                    long long mod_bs, int rows, int d, float eps) {
+                                                                    long long mod_bs, int rows, int d, float eps, Fp8Out fo = Fp8Out{}) {
   constexpr int kWarps = kThreads / 32;
   __shared__ float red[2][kR][kWarps];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
@@ -270,19 +388,58 @@ __global__ void __launch_bounds__(kThreads) ln_modulate_rows_kernel(const __nv_b
     rstd[r] = rsqrtf(v / (float)d + eps);
   }
   __nv_bfloat16* ob = out + (long long)b * o_bs;
+  float amax[kR], inv[kR];
 #pragma unroll
-  for (int r = 0; r < kR; ++r) {
-    if (r0 + r >= rows) break;
-    uint4* op = reinterpret_cast<uint4*>(ob + (long long)(r0 + r) * o_rs);
+  for (int r = 0; r < kR; ++r) amax[r] = inv[r] = 0.f;
+#pragma unroll 1
+  for (int pass = kFp8 ? 0 : 1; pass < 2; ++pass) {
+    if (kFp8 && pass == 1) {  // red[0] is free again: every thread read it before the variance barrier
 #pragma unroll
-    for (int i = 0; i < kChunks; ++i) {
-      float f[8];
-      unpack8(buf[r][i], f);
-      const float s[8] = {sc[i][0].x, sc[i][0].y, sc[i][0].z, sc[i][0].w, sc[i][1].x, sc[i][1].y, sc[i][1].z, sc[i][1].w};
-      const float h[8] = {sh[i][0].x, sh[i][0].y, sh[i][0].z, sh[i][0].w, sh[i][1].x, sh[i][1].y, sh[i][1].z, sh[i][1].w};
+      for (int r = 0; r < kR; ++r) {
+        const float m = warp_max(amax[r]);
+        if (lane == 0) red[0][r][warp] = m;
+      }
+      __syncthreads();
 #pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean[r]) * rstd[r] * (1.f + s[j]) + h[j];
-      op[t + kThreads * i] = pack8(f);
+      for (int r = 0; r < kR; ++r) {
+        float m = 0.f;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) m = fmaxf(m, red[0][r][w]);
+        amax[r] = m;
+        inv[r] = fp8_inv_scale(m);
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < kR; ++r) {
+      if (r0 + r >= rows) break;
+      uint4* op = reinterpret_cast<uint4*>(ob + (long long)(r0 + r) * o_rs);
+#pragma unroll
+      for (int i = 0; i < kChunks; ++i) {
+        float f[8];
+        unpack8(buf[r][i], f);
+        const float s[8] = {sc[i][0].x, sc[i][0].y, sc[i][0].z, sc[i][0].w, sc[i][1].x, sc[i][1].y, sc[i][1].z, sc[i][1].w};
+        const float h[8] = {sh[i][0].x, sh[i][0].y, sh[i][0].z, sh[i][0].w, sh[i][1].x, sh[i][1].y, sh[i][1].z, sh[i][1].w};
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[j] = (f[j] - mean[r]) * rstd[r] * (1.f + s[j]) + h[j];
+        if constexpr (kFp8) {
+          round_bf16x8(f);
+          if (pass == 0) {
+            amax[r] = absmax8(f, amax[r]);
+          } else {
+            uint2* qp = reinterpret_cast<uint2*>(fo.q + (long long)b * fo.q_bs + (long long)(r0 + r) * fo.q_rs);
+            qp[t + kThreads * i] = e4m3x8(f, inv[r]);
+          }
+        } else {
+          op[t + kThreads * i] = pack8(f);
+        }
+      }
+    }
+  }
+  if constexpr (kFp8) {
+    if (t == 0) {
+#pragma unroll
+      for (int r = 0; r < kR; ++r)
+        if (r0 + r < rows) fo.scale[(long long)b * fo.s_bs + r0 + r] = fp8_row_scale(amax[r]);
     }
   }
 }
@@ -787,7 +944,9 @@ static int launch_ln_modulate(const void* x, int64_t x_rs, int64_t x_bs, void* o
                               const float* shift, const float* scale, int64_t mod_bs, int32_t batch, int32_t rows, int32_t d,
                               float eps, const int32_t* slot_token, int32_t capacity, int32_t tokens_per_batch,
                               int32_t empty_index, int64_t mod_es, void* stream, const char* name,
-                              ug::RowSegs segs = ug::RowSegs{0, {0}}, int64_t mod_seg_stride = 0) {
+                              ug::RowSegs segs = ug::RowSegs{0, {0}}, int64_t mod_seg_stride = 0,
+                              ug::Fp8Out fo = ug::Fp8Out{nullptr, 0, 0, nullptr, 0}) {
+  const bool fp8 = fo.q != nullptr;  // ln_modulate_fp8: e4m3 rows + scales instead of `out` (same kernel choice, same bits)
   UG_CHECK_ARG(x && out && shift && scale, "%s: null pointer", name);
   UG_CHECK_ARG(batch >= 1 && rows >= 1 && d >= 8 && d % 8 == 0, "%s: bad shape batch %d rows %d d %d", name, batch, rows, d);
   UG_CHECK_ARG(x_rs % 8 == 0 && o_rs % 8 == 0 && x_bs % 8 == 0 && o_bs % 8 == 0 && mod_bs % 4 == 0 && mod_es % 4 == 0 &&
@@ -809,23 +968,38 @@ static int launch_ln_modulate(const void* x, int64_t x_rs, int64_t x_bs, void* o
     const dim3 g((unsigned)((rows + kR - 1) / kR), (unsigned)batch);
     const int nvec = d >> 3;
     bool done = true;
-    if (ln_kernel_choice() == 2 && nvec == 3 * 128 && (long long)g.x * batch > 2LL * num_sms()) {
+    // (the persistent kernel is bit-identical to the one-group-per-block kernel: the fp8 form uses the latter)
+    if (!fp8 && ln_kernel_choice() == 2 && nvec == 3 * 128 && (long long)g.x * batch > 2LL * num_sms()) {
       // persistent: two blocks per SM over all samples, each walking its row groups with the next group's rows in flight
       const dim3 gp((unsigned)std::max(1, std::min((int)g.x, (2 * num_sms() + batch - 1) / batch)), (unsigned)batch);
       ln_modulate_stream_kernel<128, 3, kR><<<gp, 128, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps);
     } else
-    if (nvec == 3 * 128) ln_modulate_rows_kernel<128, 3, kR><<<g, 128, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps);
-    else if (nvec == 3 * 64) ln_modulate_rows_kernel<64, 3, kR><<<g, 64, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps);
-    else if (nvec == 2 * 128) ln_modulate_rows_kernel<128, 2, kR><<<g, 128, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps);
+#define UG_LN_ROWS(T, C)                                                                                                 \
+  do {                                                                                                                   \
+    if (fp8) ln_modulate_rows_kernel<T, C, kR, true><<<g, T, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps, fo); \
+    else ln_modulate_rows_kernel<T, C, kR><<<g, T, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, rows, d, eps);            \
+  } while (0)
+    if (nvec == 3 * 128) UG_LN_ROWS(128, 3);
+    else if (nvec == 3 * 64) UG_LN_ROWS(64, 3);
+    else if (nvec == 2 * 128) UG_LN_ROWS(128, 2);
     else done = false;
+#undef UG_LN_ROWS
     if (done) {
       UG_CHECK_LAUNCH(name);
       return UG_OK;
     }
   }
-#define UG_LN_LAUNCH(V) ln_modulate_kernel<V><<<grid, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride)
+#define UG_LN_LAUNCH(V)                                                                                                           \
+  do {                                                                                                                            \
+    if (fp8) ln_modulate_kernel<V, true><<<grid, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride, fo); \
+    else ln_modulate_kernel<V><<<grid, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride); \
+  } while (0)
   const int grid2 = (int)((warps + 3) / 4);  // two warps per row, four rows per 256-thread block
-#define UG_LN2_LAUNCH(V) ln_modulate2_kernel<V><<<grid2, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride)
+#define UG_LN2_LAUNCH(V)                                                                                                          \
+  do {                                                                                                                            \
+    if (fp8) ln_modulate2_kernel<V, true><<<grid2, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride, fo); \
+    else ln_modulate2_kernel<V><<<grid2, block, 0, s>>>(xp, x_rs, x_bs, op, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, slot_token, capacity, tokens_per_batch, empty_index, mod_es, segs, mod_seg_stride); \
+  } while (0)
   if (d <= 8 * 32 * 2) UG_LN_LAUNCH(2);
   else if (d <= 8 * 64 * 3) UG_LN2_LAUNCH(3);
   else if (d <= 8 * 64 * 6) UG_LN2_LAUNCH(6);
@@ -842,6 +1016,41 @@ extern "C" int ug_ln_modulate(const void* x, int64_t x_rs, int64_t x_bs, void* o
                               int32_t d, float eps, void* stream) {
   return launch_ln_modulate(x, x_rs, x_bs, out, o_rs, o_bs, shift, scale, mod_bs, batch, rows, d, eps, nullptr, 1, 1, 0, 0, stream,
                             "ln_modulate");
+}
+
+extern "C" int ug_ln_modulate_fp8(const void* x, int64_t x_rs, int64_t x_bs, void* q, int64_t q_rs, int64_t q_bs, float* q_scale,
+                                  int64_t q_scale_bs, const float* shift, const float* scale, int64_t mod_bs, int32_t batch,
+                                  int32_t rows, int32_t d, float eps, void* stream) {
+  UG_CHECK_ARG(q && q_scale, "ln_modulate_fp8: null output pointer");
+  UG_CHECK_ARG((reinterpret_cast<uintptr_t>(q) & 7) == 0 && q_rs % 8 == 0 && q_bs % 8 == 0 && (reinterpret_cast<uintptr_t>(q_scale) & 3) == 0,
+               "ln_modulate_fp8: e4m3 rows must be 8-byte aligned");
+  UG_CHECK_ARG(batch == 1 || q_bs >= (int64_t)rows * q_rs, "ln_modulate_fp8: overlapping output batches");
+  // `out` is never written in the fp8 form: the input pointer stands in for it in the shared argument checks
+  return launch_ln_modulate(x, x_rs, x_bs, const_cast<void*>(x), x_rs, x_bs, shift, scale, mod_bs, batch, rows, d, eps, nullptr, 1, 1,
+                            0, 0, stream, "ln_modulate_fp8", ug::RowSegs{0, {0}}, 0,
+                            ug::Fp8Out{static_cast<uint8_t*>(q), q_rs, q_bs, q_scale, q_scale_bs});
+}
+
+extern "C" int ug_quant_rows_fp8(const void* x, int64_t x_rs, int64_t x_bs, void* q, int64_t q_rs, int64_t q_bs, float* scale,
+                                 int64_t scale_bs, int32_t batch, int32_t rows, int32_t k, void* stream) {
+  UG_CHECK_ARG(x && q && scale, "quant_rows_fp8: null pointer");
+  UG_CHECK_ARG(batch >= 1 && batch <= 65535 && rows >= 1 && k >= 8 && k % 8 == 0, "quant_rows_fp8: bad shape batch %d rows %d k %d",
+               batch, rows, k);
+  UG_CHECK_ARG(aligned16(x) && x_rs % 8 == 0 && x_bs % 8 == 0 && (reinterpret_cast<uintptr_t>(q) & 7) == 0 && q_rs % 8 == 0 &&
+                   q_bs % 8 == 0 && (reinterpret_cast<uintptr_t>(scale) & 3) == 0,
+               "quant_rows_fp8: bf16 rows must be 16-byte, e4m3 rows 8-byte aligned");
+  if (k > 8 * 256 * 8) {
+    set_error("quant_rows_fp8: k = %d exceeds the register-resident row limit (16384)", k);
+    return UG_ERR_UNSUPPORTED;
+  }
+  auto s = reinterpret_cast<cudaStream_t>(stream);
+  const ug::Fp8Out o{static_cast<uint8_t*>(q), q_rs, q_bs, scale, scale_bs};
+  const dim3 g((unsigned)rows, (unsigned)batch);
+  auto xp = (const __nv_bfloat16*)x;
+  if (k <= 8 * 128 * 4) quant_rows_fp8_kernel<128, 4><<<g, 128, 0, s>>>(xp, x_rs, x_bs, o, k);
+  else quant_rows_fp8_kernel<256, 8><<<g, 256, 0, s>>>(xp, x_rs, x_bs, o, k);
+  UG_CHECK_LAUNCH("quant_rows_fp8");
+  return UG_OK;
 }
 
 extern "C" int ug_ln_modulate_segs(const void* x, int64_t x_rs, int64_t x_bs, void* out, int64_t o_rs, int64_t o_bs,

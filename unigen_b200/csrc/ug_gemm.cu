@@ -1,5 +1,7 @@
 // Dense bf16 GEMM for sm_100a: TMA -> 128B-swizzled smem ring -> tcgen05.mma (accumulators in TMEM,
 // double-buffered) -> fused epilogue from TMEM (bias / GELU-tanh / gate * alpha / residual) -> HBM.
+// kFp8 instances read e4m3 operands (kind::f8f6f4, one 128-byte swizzle row = 128 elements, so stage bytes, TMA boxes and
+// smem descriptors keep their sizes) and dequantise the accumulator with per-row / per-channel scales before the epilogue.
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM owner), warps 2..9 = epilogue
 // (warp w reads TMEM lanes 32*(w%4)..+31, the hardware lane-quarter rule of tcgen05.ld; the two warps that share a lane
@@ -55,6 +57,11 @@ struct GemmParams {
   // block is the box of the tile's 128 output pixels shifted by the tap offset (out-of-image pixels arrive as zeros from the
   // TMA unit: the padding costs nothing). conv_cblocks == 0: plain GEMM.
   int conv_cblocks, conv_w;
+  // row-wise fp8 dequantisation (kFp8 instances): acc[r, c] * a_scale[b, r] * w_scale[wb, c]
+  const float* a_scale;
+  long long a_scale_bs;
+  const float* w_scale;
+  long long w_scale_bs;
 };
 
 // host-side description of the convolution a GEMM launch computes (ug_conv3x3_bf16)
@@ -63,13 +70,14 @@ struct ConvDesc {
   int batch, h, w, c_in;
 };
 
-template <int kCta, int BN, int kStages, bool kTmaEpi = false>
+template <int kCta, int BN, int kStages, bool kTmaEpi = false, bool kFp8 = false>
 struct GemmCfg {
   static constexpr int BM = 128;  // rows per CTA
-  static constexpr int BK = 64;   // 64 bf16 = one 128-byte swizzle row
+  static constexpr int ESIZE = kFp8 ? 1 : 2;
+  static constexpr int BK = 128 / ESIZE;  // 64 bf16 / 128 e4m3 = one 128-byte swizzle row
   static constexpr int BN_LOAD = BN / kCta;
-  static constexpr int A_BYTES = BM * BK * 2;
-  static constexpr int B_BYTES = BN_LOAD * BK * 2;
+  static constexpr int A_BYTES = BM * BK * ESIZE;
+  static constexpr int B_BYTES = BN_LOAD * BK * ESIZE;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int TMEM_COLS = 2 * BN;
   // smem-staged epilogue: every epilogue warp owns EPI_SLABS staging slabs of 32 rows x 64 bf16 columns (4 KB, 128B-swizzled:
@@ -98,6 +106,24 @@ __device__ __forceinline__ int seg_index_of(const GemmParams& p, int r) {
   for (int s = 0; s < p.lora_nseg; ++s)
     if (r >= p.lora_bounds[s] && r < p.lora_bounds[s + 1]) g = s;
   return g;
+}
+
+// fp8: dequantise the 32 accumulator columns [col0, col0 + 32) of one row in place, acc * a_scale(row) * w_scale[c]; this comes
+// before every other epilogue op. Columns past n (partial last tile) read no scale and are never stored.
+__device__ __forceinline__ void dequant32(const GemmParams& p, uint32_t (&v)[32], int b, float a_s, int col0) {
+  const float* ws = p.w_scale + (p.w_batched ? (long long)b * p.w_scale_bs : 0LL);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int c = col0 + 8 * j;
+    float4 w0 = make_float4(0.f, 0.f, 0.f, 0.f), w1 = w0;
+    if (c < p.n) {
+      w0 = __ldg(reinterpret_cast<const float4*>(ws + c));
+      w1 = __ldg(reinterpret_cast<const float4*>(ws + c + 4));
+    }
+    const float w[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[8 * j + i] = __float_as_uint(__uint_as_float(v[8 * j + i]) * a_s * w[i]);
+  }
 }
 
 __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32_t (&v)[32], int b, int r, int col0,
@@ -339,12 +365,12 @@ __device__ __forceinline__ void tile_coords(const GemmParams& p, int tile, int m
   nt = in_band / size;
 }
 
-template <int kCta, int BN, int kStages, bool kTmaEpi>
+template <int kCta, int BN, int kStages, bool kTmaEpi, bool kFp8>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
                  const __grid_constant__ CUtensorMap tma_a2, const __grid_constant__ CUtensorMap tma_w2,
                  const __grid_constant__ CUtensorMap tma_c, const __grid_constant__ CUtensorMap tma_r, const GemmParams p) {
-  using Cfg = GemmCfg<kCta, BN, kStages, kTmaEpi>;
+  using Cfg = GemmCfg<kCta, BN, kStages, kTmaEpi, kFp8>;
   extern __shared__ uint8_t smem_raw[];
   // 128B swizzle atoms need 1024-byte alignment; the offset is identical in both CTAs of a pair.
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -451,7 +477,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   } else if (warp == 1) {
     // ------------------------------ MMA issuer (leader CTA only) ------------------------------
     if (cta_rank == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(Cfg::BM * kCta, BN, false, false);
+      constexpr uint32_t idesc = kFp8 ? make_idesc_e4m3(Cfg::BM * kCta, BN) : make_idesc_bf16(Cfg::BM * kCta, BN, false, false);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -470,9 +496,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             const uint64_t a_desc = make_sdesc_sw128(smem_u32(smem_a + stage * Cfg::A_BYTES), 16, 1024);
             const uint64_t b_desc = make_sdesc_sw128(smem_u32(smem_b + stage * Cfg::B_BYTES), 16, 1024);
 #pragma unroll
-            for (int k = 0; k < Cfg::BK / 16; ++k) {
-              // +32 bytes per K=16 step inside the 128-byte swizzle row (start-address field is in 16 B units)
-              umma_ss<kCta>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
+            for (int k = 0; k < 4; ++k) {
+              // +32 bytes per K step (16 bf16 / 32 e4m3) inside the 128-byte swizzle row (start-address field is in 16 B units)
+              umma_ss<kCta, kFp8>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
             }
             if constexpr (kCta == 1) {
               umma_commit(&empty[stage]);
@@ -509,6 +535,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
       }
       const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + as * BN;
       const int lora_g = (p.lora_t || p.colmask_block) ? lora_group_of(p, r) : -1;
+      // fp8: this row's activation scale (rows past the matrix edge are computed, never stored: read a valid entry)
+      const float a_s = kFp8 ? __ldg(p.a_scale + (long long)b * p.a_scale_bs + min(r, p.rows - 1)) : 1.f;
+      (void)a_s;
       // gate vector of this row: per sample, and per row segment when gate_seg_stride is set (once per tile, not per chunk)
       const float* gate_row = p.gate ? p.gate + (long long)b * p.gate_bs + (p.gate_seg_stride ? seg_index_of(p, r) * p.gate_seg_stride : 0)
                                      : nullptr;
@@ -560,6 +589,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
               uint32_t v[32];
               tmem_ld_32x32(taddr + (ch0 + ch) * 32, v);
               tmem_ld_wait();
+              if constexpr (kFp8) dequant32(p, v, b, a_s, cw0 + 32 * ch);
               if (cw0 + 32 * ch < p.n) ss[(p.qk_dh == 64) ? (ch >> 1) : 0] += chunk_sumsq(p, v, b, cw0 + 32 * ch);
             }
             if (p.qk_dh != 64) ss[1] = ss[0];
@@ -581,6 +611,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             uint32_t v[32];
             tmem_ld_32x32(taddr + (ch0 + 2 * sl + h) * 32, v);
             tmem_ld_wait();
+            if constexpr (kFp8) dequant32(p, v, b, a_s, cs0 + 32 * h);
             if (sl == Cfg::EPI_SLABS - 1 && h == 1) release_acc();
             if (active) {
 #pragma unroll
@@ -627,6 +658,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
               uint32_t v[32];
               tmem_ld_32x32(taddr + c_h + ch * 32, v);
               tmem_ld_wait();
+              if constexpr (kFp8) dequant32(p, v, b, a_s, col_h + ch * 32);
               ss += chunk_sumsq(p, v, b, col_h + ch * 32);
             }
             rstd = rsqrtf(ss / (float)p.qk_dh + p.qk_eps);
@@ -636,6 +668,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             uint32_t v[32];
             tmem_ld_32x32(taddr + c_h + ch * 32, v);
             tmem_ld_wait();
+            if constexpr (kFp8) dequant32(p, v, b, a_s, col_h + ch * 32);
             if (c_h + p.qk_dh >= c_hi && ch == cph - 1) release_acc();
             if (r < p.rows && active) epilogue_qkv_chunk(p, v, b, r, col_h + ch * 32, ch * 32, which, rstd);
           }
@@ -650,6 +683,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           tmem_ld_wait();
           if (ch == ch0 + kChunksPerWarp - 1) release_acc();
           const int col0 = n0 + ch * 32;
+          if constexpr (kFp8) dequant32(p, v, b, a_s, col0);
           if (p.colmask_block && col0 / p.colmask_block != lora_g) {
             // grouped down-projection: a row keeps only the column block of its own adapter group
 #pragma unroll
@@ -672,10 +706,17 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   }
 }
 
-template <int kCta, int BN, int kStages, bool kTmaEpi = false>
-static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDesc* conv = nullptr) {
-  using Cfg = GemmCfg<kCta, BN, kStages, kTmaEpi>;
-  auto kern = gemm_bf16_kernel<kCta, BN, kStages, kTmaEpi>;
+template <int kCta, int BN, int kStages, bool kTmaEpi = false, bool kFp8 = false>
+static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDesc* conv = nullptr,
+                       const ug_gemm_fp8_scales* scales = nullptr) {
+  using Cfg = GemmCfg<kCta, BN, kStages, kTmaEpi, kFp8>;
+  constexpr uint64_t E = Cfg::ESIZE;
+  // A / W operand maps: bf16, or one e4m3 per byte (UINT8) for the fp8 instances
+  auto encode_op = [](CUtensorMap* m, const void* base, int rank, const uint64_t* dims, const uint64_t* strides, const uint32_t* box) {
+    return kFp8 ? encode_tmap(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, base, rank, dims, strides, box)
+                : encode_tmap_bf16(m, base, rank, dims, strides, box);
+  };
+  auto kern = gemm_bf16_kernel<kCta, BN, kStages, kTmaEpi, kFp8>;
   static bool attr_done[64] = {false};
   if (int st = ensure_dynamic_smem(kern, Cfg::SMEM_BYTES, attr_done, "gemm"); st != UG_OK) return st;
   CUtensorMap tma_a, tma_w;
@@ -691,18 +732,18 @@ static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDes
   } else {
     uint64_t dims[3] = {(uint64_t)a.k, (uint64_t)a.rows, (uint64_t)a.batch};
     uint64_t bs = a.batch > 1 ? (uint64_t)a.a_batch_stride : (uint64_t)a.rows * a.a_row_stride;
-    uint64_t strides[2] = {(uint64_t)a.a_row_stride * 2, bs * 2};
+    uint64_t strides[2] = {(uint64_t)a.a_row_stride * E, bs * E};
     uint32_t box[3] = {(uint32_t)Cfg::BK, (uint32_t)Cfg::BM, 1};
-    int st = encode_tmap_bf16(&tma_a, a.a, 3, dims, strides, box);
+    int st = encode_op(&tma_a, a.a, 3, dims, strides, box);
     if (st != UG_OK) return st;
   }
   const bool w_batched = a.w_batch_stride != 0 && a.batch > 1;
   {
     uint64_t dims[3] = {(uint64_t)a.k, (uint64_t)a.n, (uint64_t)(w_batched ? a.batch : 1)};
     uint64_t bs = w_batched ? (uint64_t)a.w_batch_stride : (uint64_t)a.n * a.w_row_stride;
-    uint64_t strides[2] = {(uint64_t)a.w_row_stride * 2, bs * 2};
+    uint64_t strides[2] = {(uint64_t)a.w_row_stride * E, bs * E};
     uint32_t box[3] = {(uint32_t)Cfg::BK, (uint32_t)Cfg::BN_LOAD, 1};
-    int st = encode_tmap_bf16(&tma_w, a.w, 3, dims, strides, box);
+    int st = encode_op(&tma_w, a.w, 3, dims, strides, box);
     if (st != UG_OK) return st;
   }
   CUtensorMap tma_a2 = tma_a, tma_w2 = tma_w;
@@ -750,12 +791,12 @@ static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDes
   p.n_tiles = (a.n + BN - 1) / BN;
   {
     // A bytes one sweep over all m-tiles touches; above ~40 MB it no longer survives in the 126 MB L2 between n-waves
-    const long long a_bytes = (long long)a.batch * a.rows * (a.k + (a.a2 ? a.k2 : 0)) * 2;
+    const long long a_bytes = (long long)a.batch * a.rows * (a.k + (a.a2 ? a.k2 : 0)) * Cfg::ESIZE;
     const int mb_all = p.m_tiles * a.batch;
     p.group_m = mb_all;
     if (a_bytes > (40LL << 20) && !(a.w_batch_stride != 0 && a.batch > 1)) {
       // band of A row-tiles worth ~24 MB: it stays in L2 while the band sweeps every n-tile, so A is read from HBM once
-      const long long tile_bytes = (long long)Cfg::BM * kCta * (a.k + (a.a2 ? a.k2 : 0)) * 2;
+      const long long tile_bytes = (long long)Cfg::BM * kCta * (a.k + (a.a2 ? a.k2 : 0)) * Cfg::ESIZE;
       long long gm = (24LL << 20) / tile_bytes;
       gm = gm < 2 ? 2 : (gm > 16 ? 16 : gm);
       p.group_m = gm < mb_all ? (int)gm : mb_all;
@@ -779,6 +820,10 @@ static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDes
   p.lora_r = a.lora_rank; p.lora_block_n = a.lora_block_n > 0 ? a.lora_block_n : a.n; p.lora_nseg = a.lora_nseg;
   for (int i = 0; i <= UG_MAX_SEGMENTS; ++i) p.lora_bounds[i] = i <= a.lora_nseg ? a.lora_seg_bounds[i] : a.rows;
   for (int i = 0; i < UG_MAX_SEGMENTS; ++i) p.lora_group[i] = i < a.lora_nseg ? a.lora_seg_group[i] : -1;
+  p.a_scale = scales ? scales->a_scale : nullptr;
+  p.a_scale_bs = scales ? scales->a_scale_batch_stride : 0;
+  p.w_scale = scales ? scales->w_scale : nullptr;
+  p.w_scale_bs = scales ? scales->w_scale_batch_stride : 0;
 
   const int sms = num_sms();
   int units = kCta == 2 ? sms / 2 : sms;
@@ -832,16 +877,43 @@ static int pick_tile_variant(int batch, int rows, int n) {
   return variant;
 }
 
-}  // namespace ug
+template <bool kFp8>
+static int launch_variant(int variant, const ug_gemm_args& a, cudaStream_t s, const ug_gemm_fp8_scales* scales) {
+  switch (variant) {
+    case 1: return launch_gemm<1, 256, 4, false, kFp8>(a, s, nullptr, scales);
+    case 2: return launch_gemm<2, 256, 6, false, kFp8>(a, s, nullptr, scales);
+    case 3: return launch_gemm<1, 128, 6, false, kFp8>(a, s, nullptr, scales);
+    case 4: return launch_gemm<2, 256, 5, true, kFp8>(a, s, nullptr, scales);
+    case 5: return launch_gemm<1, 256, 3, true, kFp8>(a, s, nullptr, scales);
+    case 6: return launch_gemm<1, 128, 6, true, kFp8>(a, s, nullptr, scales);
+    default:
+      set_error("gemm: unknown variant %d", a.variant);
+      return UG_ERR_INVALID;
+  }
+}
 
-extern "C" int ug_gemm_bf16(const ug_gemm_args* args, void* stream) {
-  using namespace ug;
+// ug_gemm_bf16 (scales == NULL) and ug_gemm_fp8: argument checks, tile / epilogue choice, launch
+static int gemm_entry(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream) {
+  const bool fp8 = scales != nullptr;
   UG_CHECK_ARG(args != nullptr, "gemm: null args");
   const ug_gemm_args& a = *args;
   UG_CHECK_ARG(a.a && a.w && a.c, "gemm: null operand pointer");
   UG_CHECK_ARG(a.batch >= 1 && a.rows >= 1 && a.n >= 1 && a.k >= 1, "gemm: empty problem (batch %d rows %d n %d k %d)",
                a.batch, a.rows, a.n, a.k);
   UG_CHECK_ARG(a.k % 8 == 0 && a.n % 8 == 0, "gemm: n (%d) and k (%d) must be multiples of 8", a.n, a.k);
+  if (fp8) {
+    // e4m3 rows: TMA strides must be multiples of 16 bytes = 16 elements
+    UG_CHECK_ARG(a.k % 16 == 0, "gemm_fp8: k (%d) must be a multiple of 16", a.k);
+    UG_CHECK_ARG(a.a_row_stride % 16 == 0 && a.w_row_stride % 16 == 0 && (a.batch == 1 || a.a_batch_stride % 16 == 0) &&
+                     a.w_batch_stride % 16 == 0,
+                 "gemm_fp8: e4m3 row / batch strides must be multiples of 16 elements (16 bytes)");
+    UG_CHECK_ARG(!a.lora_t && !a.colmask_block && !a.a2 && !a.w2,
+                 "gemm_fp8: lora_t, colmask_block and the second operand pair (a2 / w2) are bf16-only");
+    UG_CHECK_ARG(scales->a_scale && scales->w_scale, "gemm_fp8: null a_scale / w_scale");
+    UG_CHECK_ARG((reinterpret_cast<uintptr_t>(scales->a_scale) & 3) == 0 && (reinterpret_cast<uintptr_t>(scales->w_scale) & 15) == 0 &&
+                     scales->w_scale_batch_stride % 4 == 0,
+                 "gemm_fp8: w_scale must be 16-byte aligned (batch stride a multiple of 4), a_scale 4-byte aligned");
+  }
   UG_CHECK_ARG(a.a_row_stride % 8 == 0 && a.w_row_stride % 8 == 0 && a.c_row_stride % 8 == 0,
                "gemm: row strides must be multiples of 8 elements (16 bytes)");
   UG_CHECK_ARG(a.a_row_stride >= a.k && a.w_row_stride >= a.k && a.c_row_stride >= a.n, "gemm: row stride smaller than row");
@@ -916,17 +988,21 @@ extern "C" int ug_gemm_bf16(const ug_gemm_args* args, void* stream) {
                  "gemm: the staged fused QK-norm epilogue needs a 256-column tile (variants 4 / 5) and qk_d a multiple of 128");
     UG_CHECK_ARG(!a.residual || a.res_batch_stride % 8 == 0 || a.batch == 1, "gemm: residual batch stride must be a multiple of 8");
   }
-  switch (variant) {
-    case 1: return launch_gemm<1, 256, 4>(a, s);
-    case 2: return launch_gemm<2, 256, 6>(a, s);
-    case 3: return launch_gemm<1, 128, 6>(a, s);
-    case 4: return launch_gemm<2, 256, 5, true>(a, s);
-    case 5: return launch_gemm<1, 256, 3, true>(a, s);
-    case 6: return launch_gemm<1, 128, 6, true>(a, s);
-    default:
-      set_error("gemm: unknown variant %d", a.variant);
-      return UG_ERR_INVALID;
+  return fp8 ? launch_variant<true>(variant, a, s, scales) : launch_variant<false>(variant, a, s, nullptr);
+}
+
+}  // namespace ug
+
+extern "C" int ug_gemm_bf16(const ug_gemm_args* args, void* stream) { return ug::gemm_entry(args, nullptr, stream); }
+
+// Row-wise fp8 GEMM: the persistent kernel above instantiated for e4m3 operands (kind::f8f6f4) with the dequantisation
+// multiply in front of every epilogue path. An opt-in path of `UniGenFlux.quantize_fp8()`.
+extern "C" int ug_gemm_fp8(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream) {
+  if (scales == nullptr) {
+    ug::set_error("gemm_fp8: null scales");
+    return UG_ERR_INVALID;
   }
+  return ug::gemm_entry(args, scales, stream);
 }
 
 // 3x3 convolution, stride 1, zero padding 1, over NHWC bf16 images as an implicit GEMM on the tcgen05 path above: no im2col

@@ -49,8 +49,8 @@ static encode_fn_t get_encode_fn() {
   return fn;
 }
 
-int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
-                     const uint64_t* strides_bytes, const uint32_t* box) {
+int encode_tmap(CUtensorMap* map, CUtensorMapDataType dtype, const void* base, int rank, const uint64_t* dims,
+                const uint64_t* strides_bytes, const uint32_t* box) {
   encode_fn_t fn = get_encode_fn();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled driver entry point not available");
@@ -75,7 +75,7 @@ int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_
       }
     }
   }
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gdims, gstrides,
+  CUresult r = fn(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), gdims, gstrides,
                   gbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -85,6 +85,11 @@ int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_
     return UG_ERR_CUDA;
   }
   return UG_OK;
+}
+
+int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                     const uint32_t* box) {
+  return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, base, rank, dims, strides_bytes, box);
 }
 
 }  // namespace ug

@@ -36,6 +36,9 @@ int ensure_dynamic_smem(Kernel kern, int bytes, bool (&done)[64], const char* na
 // BYTES for dims 1..rank-1. Returns UG_OK or an error status (message set).
 int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                      const uint32_t* box);
+// Same with any element type (the fp8 GEMM's operands are UINT8 maps: one e4m3 per byte, 128 elements per swizzle row).
+int encode_tmap(CUtensorMap* map, CUtensorMapDataType dtype, const void* base, int rank, const uint64_t* dims,
+                const uint64_t* strides_bytes, const uint32_t* box);
 
 #define UG_CHECK_ARG(cond, ...)      \
   do {                               \

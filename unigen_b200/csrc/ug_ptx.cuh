@@ -200,6 +200,14 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, bool a_mn_m
          | ((uint32_t)(N >> 3) << 17)           //
          | ((uint32_t)(M >> 4) << 24);
 }
+// Instruction descriptor for kind::f8f6f4 with e4m3 A/B (format code 0) and fp32 accumulation.
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(int M, int N) {
+  return (1u << 4)                              // D format: f32
+         | (0u << 7)                            // A format: e4m3
+         | (0u << 10)                           // B format: e4m3
+         | ((uint32_t)(N >> 3) << 17)           //
+         | ((uint32_t)(M >> 4) << 24);
+}
 // One lane of the (converged) warp: ptxas knows the region guarded by elect.sync is single-threaded, so the operands of the
 // tcgen05 instructions issued there stay in uniform registers. Under `if (lane == 0)` it cannot prove that and wraps every
 // tcgen05.mma in an R2UR + ELECT / BRA.U.ANY loop (~12 scalar instructions per MMA).
@@ -210,20 +218,33 @@ __device__ __forceinline__ bool elect_one_sync() {
       : "=r"(pred));
   return pred != 0;
 }
-// D[tmem] (+)= A[smem] * B[smem]; issued by ONE thread.
-template <int kCtaGroup>
+// D[tmem] (+)= A[smem] * B[smem]; issued by ONE thread. kFp8: kind::f8f6f4 (K = 32 e4m3 per instruction), else kind::f16
+// (K = 16 bf16): both advance 32 bytes of the 128-byte swizzle row per instruction.
+template <int kCtaGroup, bool kFp8 = false>
 __device__ __forceinline__ void umma_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                         uint32_t accumulate) {
-  if constexpr (kCtaGroup == 1) {
+  if constexpr (kCtaGroup == 1 && !kFp8) {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
         "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
-  } else {
+  } else if constexpr (kCtaGroup == 2 && !kFp8) {
     asm volatile(
         "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+  } else if constexpr (kCtaGroup == 1) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+  } else {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
         "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
   }

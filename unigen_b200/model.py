@@ -29,6 +29,7 @@ from . import ops
 from .ops import UG_ACT_GELU_TANH
 
 BF16 = torch.bfloat16
+FP8 = torch.float8_e4m3fn
 
 
 class FluxArch:
@@ -75,6 +76,11 @@ class _Weights:
 
 
 class _DoubleBlockW:
+    # linears `UniGenFlux.quantize_fp8()` converts; once it has, `fp8` is True and each of them is (W e4m3 [N, K], bias bf16 [N],
+    # w_scale fp32 [N]) instead of (W bf16, bias)
+    FP8_LINEARS = ("qkv", "add_qkv", "to_out", "to_add_out", "ff1", "ff2", "ffc1", "ffc2")
+    fp8 = False
+
     def __init__(self, ws: _Weights, p: str, D: int, dh: int):
         self.norm1 = ws.linear(p + ".norm1.linear", 6 * D, D)
         self.norm1_ctx = ws.linear(p + ".norm1_context.linear", 6 * D, D)
@@ -93,6 +99,9 @@ class _DoubleBlockW:
 
 
 class _SingleBlockW:
+    FP8_LINEARS = ("qkv", "mlp", "out")
+    fp8 = False
+
     def __init__(self, ws: _Weights, p: str, D: int, dh: int):
         self.norm = ws.linear(p + ".norm.linear", 3 * D, D)
         self.qkv = ws.fused([f"{p}.attn.to_q", f"{p}.attn.to_k", f"{p}.attn.to_v"], D, D)
@@ -305,6 +314,7 @@ class UniGenFlux(_DenoiserBase):
         self.norm_out_w = ws.linear("norm_out.linear", 2 * D, D)
         # proj_out has only in_channels (64) output features: keep it as is, the GEMM masks the partial N tile
         self.proj_out_w = ws.linear("proj_out", a.in_channels, D)
+        self.linear_dtype = BF16  # float8_e4m3fn after quantize_fp8()
 
     # ---------------------------------------------------------------------------------------------------------
     # reference API: construction
@@ -359,6 +369,51 @@ class UniGenFlux(_DenoiserBase):
     def requires_grad_(self, requires_grad: bool = True):  # infer.py:143 `transformer.requires_grad_(False)`: inference-only path
         if requires_grad:
             raise ops.UgError("the B200-native path is forward-only (SURVEY.md §3.2: training is out of scope)")
+        return self
+
+    def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):
+        if self.linear_dtype != BF16:
+            raise ops.UgError("load_state_dict on an fp8-quantised model: its block linears no longer hold bf16 weights — load the "
+                              "checkpoint into a fresh model, then call quantize_fp8()")
+        return super().load_state_dict(state_dict, strict=strict, assign=assign)
+
+    def init_random_(self, seed: int = 0, zero_linear_std: Optional[float] = 0.02):
+        if self.linear_dtype != BF16:
+            raise ops.UgError("init_random_ on an fp8-quantised model: its quantised block weights are not in state_dict() any more "
+                              "and would keep their values — initialise a fresh model, then call quantize_fp8()")
+        return super().init_random_(seed=seed, zero_linear_std=zero_linear_std)
+
+    @torch.no_grad()
+    def quantize_fp8(self):
+        """Opt-in fp8 (e4m3) transformer-block linears, in place; returns self. Every linear of the base and control double
+        blocks (q|k|v, add_q|k|v, to_out, to_add_out, ff, ff_context) and single blocks (q|k|v, proj_mlp, proj_out) gets one fp32
+        scale per output channel and is stored as e4m3; its bf16 copy is released (and leaves `state_dict()`). In every forward
+        their operands are quantised per token row on the device and the GEMMs run on the fp8 tensor cores. Embedders, the
+        CoMoE pre-stage (its expert, shared-expert and consistency blocks: routing stays bit-exact), the AdaLN GEMVs, the control
+        add-linears, proj_out and attention stay bf16. Call after `from_pretrained` / `init_condition_block` and any
+        `load_state_dict`. Afterwards `state_dict()` / `parameters()` no longer list the quantised weights (their biases and every
+        bf16 tensor stay), and `load_state_dict` / `init_random_` raise `UgError`."""
+        if not self._control_ready:
+            raise ops.UgError("call init_condition_block(condition_nums=..., control_params=...) before quantize_fp8()")
+        if self.linear_dtype == FP8:
+            return self
+        views = self._ws.views
+        for w in self.double + self.ctrl_double + self.single + self.ctrl_single:
+            for name in w.FP8_LINEARS:
+                W, bias = getattr(w, name)
+                q, w_scale = ops.quant_rows_fp8(W)  # a row of W is an output channel
+                ptr = W.untyped_storage().data_ptr()
+                for k in [k for k, v in views.items() if k.endswith(".weight") and v.untyped_storage().data_ptr() == ptr]:
+                    del views[k]
+                setattr(w, name, (q, bias, w_scale))
+            w.fp8 = True
+        self.linear_dtype = FP8
+        # workspaces (and the graphs captured over them, the pipeline's whole-loop graphs included) hold bf16 operands only
+        from .pipeline import _GRAPHS_ATTR
+        self.__dict__.pop(_GRAPHS_ATTR, None)
+        self._workspaces.clear()
+        self._graphs.clear()
+        self._buf = None
         return self
 
     def init_condition_block(self, condition_nums: int = 1, **kwargs):
@@ -484,6 +539,12 @@ class UniGenFlux(_DenoiserBase):
         b.temb, b.ctemb, b.cdtemb = b.TEMBS[0], b.TEMBS[1], b.TEMBS[2]
         b.cdtemb_c = [b.TEMBS[3 + c] for c in range(self.condition_nums)]
         b.mod_plans = None
+        if self.linear_dtype == FP8:  # e4m3 operands (+ one fp32 scale per row) of the quantised block linears
+            f8 = lambda *sh: z(*sh, dt=FP8)  # noqa: E731
+            b.NXQ, b.NXS = f8(B, Smax, D), z(B, Smax, dt=torch.float32)
+            b.AOQ, b.AOS = f8(B, Smax, D), z(B, Smax, dt=torch.float32)
+            b.FFQ, b.FFS = f8(B, Smax, 4 * D), z(B, Smax, dt=torch.float32)
+            b.CATQ, b.CATS = f8(B, S, 5 * D), z(B, S, dt=torch.float32)
         if consis:  # [experts' image output | consis condition output] and the id tables of the two consis_module[0] calls
             b.CONS = z(B, 2 * N, D)
             b.ropek0 = z(2 * N, self.arch.attention_head_dim, dt=torch.float32)
@@ -592,6 +653,22 @@ class UniGenFlux(_DenoiserBase):
                 ops.qk_rmsnorm_rope(qk[:, n_ctx:], 2 * H, dh, rms_smp, rope[n_ctx:S] if rope is not None else None, heads_per_weight=H)
         return self._attend(buf, S, buf.AO[:, :S])
 
+    def _ln(self, w, x, nx, q, shift, scale):
+        """LN + modulate of a block input into the bf16 operand `nx`, or (fp8 weight set) straight into q = (e4m3, row scales)."""
+        if w.fp8:
+            ops.ln_modulate_fp8(x, q[0], q[1], shift, scale)
+        else:
+            ops.ln_modulate(x, nx, shift, scale)
+
+    def _linear(self, wl, x, q, out, quantize: bool = False, **epi):
+        """One block linear: the bf16 GEMM of x with (W, bias), or for an fp8 (W e4m3, bias, w_scale) the fp8 GEMM of
+        q = (e4m3 rows, row scales) — quantised from x first when `quantize` (operands no LN kernel produced)."""
+        if len(wl) == 3:
+            if quantize:
+                ops.quant_rows_fp8(x, q[0], q[1])
+            return ops.gemm_fp8(q[0], q[1], wl[0], wl[2], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
+        return ops.gemm(x, wl[0], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
+
     def _double_block(self, buf, w: _DoubleBlockW, mod_smp, mod_ctx, smp_in, ctx_in, smp_out, ctx_out, rope):
         """diffusers FluxTransformerBlock (SURVEY.md §A.2). smp/ctx = image-role / text-role streams ([B, n, D] views);
         outputs may alias inputs (in-place residual). ctx_out=None skips the context stream's post-attention half —
@@ -600,10 +677,14 @@ class UniGenFlux(_DenoiserBase):
         D = self.inner_dim
         B, n_smp, n_ctx = smp_in.shape[0], smp_in.shape[1], ctx_in.shape[1]
         S = n_ctx + n_smp
-        gv = self.gemm_variant
         sh_a, sc_a, g_a, sh_m, sc_m, g_m = mod_smp
         csh_a, csc_a, cg_a, csh_m, csc_m, cg_m = mod_ctx
         nx_c, nx_s = buf.NX[:, :n_ctx], buf.NX[:, n_ctx:S]
+        qn_c = qn_s = qa_c = qa_s = qf_c = qf_s = None
+        if w.fp8:  # e4m3 operands (+ one fp32 scale per row) of the same rows; the pre-stage's bf16 blocks never use them
+            qn_c, qn_s = (buf.NXQ[:, :n_ctx], buf.NXS[:, :n_ctx]), (buf.NXQ[:, n_ctx:S], buf.NXS[:, n_ctx:S])
+            qa_c, qa_s = (buf.AOQ[:, :n_ctx], buf.AOS[:, :n_ctx]), (buf.AOQ[:, n_ctx:S], buf.AOS[:, n_ctx:S])
+            qf_c, qf_s = (buf.FFQ[:, :n_ctx], buf.FFS[:, :n_ctx]), (buf.FFQ[:, n_ctx:S], buf.FFS[:, n_ctx:S])
         # The text stream's GEMMs are small (M = 512 at cfg3: 24-96 tiles for 148 SMs); issued on a second stream they run
         # beside the image stream's GEMMs (disjoint rows of NX / QKV / FF) and fill the SMs those leave idle in their last wave.
         main = torch.cuda.current_stream()
@@ -613,13 +694,13 @@ class UniGenFlux(_DenoiserBase):
             if side is not None:
                 side.wait_stream(main)
             with torch.cuda.stream(side if side is not None else main):
-                ops.ln_modulate(ctx_in, nx_c, csh_a, csc_a)
-                ops.gemm(nx_c, w.add_qkv[0], out=buf.QKV[:, :n_ctx], bias=w.add_qkv[1], variant=gv,
-                         qk_norm=self._qk_norm(w.rms_ctx, rope[:n_ctx] if rope is not None else None))
+                self._ln(w, ctx_in, nx_c, qn_c, csh_a, csc_a)
+                self._linear(w.add_qkv, nx_c, qn_c, out=buf.QKV[:, :n_ctx],
+                             qk_norm=self._qk_norm(w.rms_ctx, rope[:n_ctx] if rope is not None else None))
         if n_smp:
-            ops.ln_modulate(smp_in, nx_s, sh_a, sc_a)
-            ops.gemm(nx_s, w.qkv[0], out=buf.QKV[:, n_ctx:S], bias=w.qkv[1], variant=gv,
-                     qk_norm=self._qk_norm(w.rms, rope[n_ctx:S] if rope is not None else None))
+            self._ln(w, smp_in, nx_s, qn_s, sh_a, sc_a)
+            self._linear(w.qkv, nx_s, qn_s, out=buf.QKV[:, n_ctx:S],
+                         qk_norm=self._qk_norm(w.rms, rope[n_ctx:S] if rope is not None else None))
         if side is not None:
             main.wait_stream(side)
         ao = self._joint_attention(buf, B, n_ctx, n_smp, w.rms_ctx, w.rms, rope)
@@ -627,17 +708,17 @@ class UniGenFlux(_DenoiserBase):
             if side is not None:
                 side.wait_stream(main)
             with torch.cuda.stream(side if side is not None else main):
-                ops.gemm(ao[:, :n_ctx], w.to_add_out[0], out=ctx_out, bias=w.to_add_out[1], gate=cg_a, residual=ctx_in, variant=gv)
-                ops.ln_modulate(ctx_out, nx_c, csh_m, csc_m)
-                ops.gemm(nx_c, w.ffc1[0], out=buf.FF[:, :n_ctx], bias=w.ffc1[1], act=UG_ACT_GELU_TANH, variant=gv)
-                ops.gemm(buf.FF[:, :n_ctx], w.ffc2[0], out=ctx_out, bias=w.ffc2[1], gate=cg_m, residual=ctx_out, variant=gv)
+                self._linear(w.to_add_out, ao[:, :n_ctx], qa_c, out=ctx_out, quantize=True, gate=cg_a, residual=ctx_in)
+                self._ln(w, ctx_out, nx_c, qn_c, csh_m, csc_m)
+                self._linear(w.ffc1, nx_c, qn_c, out=buf.FF[:, :n_ctx], act=UG_ACT_GELU_TANH)
+                self._linear(w.ffc2, buf.FF[:, :n_ctx], qf_c, out=ctx_out, quantize=True, gate=cg_m, residual=ctx_out)
         if n_smp:
             # h = h + gate_msa * to_out(attn)
-            ops.gemm(ao[:, n_ctx:S], w.to_out[0], out=smp_out, bias=w.to_out[1], gate=g_a, residual=smp_in, variant=gv)
+            self._linear(w.to_out, ao[:, n_ctx:S], qa_s, out=smp_out, quantize=True, gate=g_a, residual=smp_in)
             # h = h + gate_mlp * ff(LN(h) * (1 + scale_mlp) + shift_mlp)
-            ops.ln_modulate(smp_out, nx_s, sh_m, sc_m)
-            ops.gemm(nx_s, w.ff1[0], out=buf.FF[:, n_ctx:S], bias=w.ff1[1], act=UG_ACT_GELU_TANH, variant=gv)
-            ops.gemm(buf.FF[:, n_ctx:S], w.ff2[0], out=smp_out, bias=w.ff2[1], gate=g_m, residual=smp_out, variant=gv)
+            self._ln(w, smp_out, nx_s, qn_s, sh_m, sc_m)
+            self._linear(w.ff1, nx_s, qn_s, out=buf.FF[:, n_ctx:S], act=UG_ACT_GELU_TANH)
+            self._linear(w.ff2, buf.FF[:, n_ctx:S], qf_s, out=smp_out, quantize=True, gate=g_m, residual=smp_out)
         if side is not None:
             main.wait_stream(side)
 
@@ -655,15 +736,15 @@ class UniGenFlux(_DenoiserBase):
         a = self.arch
         H, dh, D = a.num_attention_heads, a.attention_head_dim, self.inner_dim
         B, S = x_in.shape[0], x_in.shape[1]
-        gv = self.gemm_variant
         shift, scale, gate = mod
         nx, cat = buf.NX[:, :S], buf.CAT[:, :S]
-        ops.ln_modulate(x_in, nx, shift, scale)
-        ops.gemm(nx, w.qkv[0], out=buf.QKV[:, :S], bias=w.qkv[1], variant=gv,
-                 qk_norm=self._qk_norm(w.rms, rope[:S] if rope is not None else None))
-        ops.gemm(nx, w.mlp[0], out=cat[:, :, D:], bias=w.mlp[1], act=UG_ACT_GELU_TANH, variant=gv)
+        qn = (buf.NXQ[:, :S], buf.NXS[:, :S]) if w.fp8 else None  # one quantised operand for both GEMMs that read nx
+        qc = (buf.CATQ[:, :S], buf.CATS[:, :S]) if w.fp8 else None
+        self._ln(w, x_in, nx, qn, shift, scale)
+        self._linear(w.qkv, nx, qn, out=buf.QKV[:, :S], qk_norm=self._qk_norm(w.rms, rope[:S] if rope is not None else None))
+        self._linear(w.mlp, nx, qn, out=cat[:, :, D:], act=UG_ACT_GELU_TANH)
         self._single_attention(buf, S, w.rms, rope, cat[:, :, :D])
-        ops.gemm(cat, w.out[0], out=x_out, bias=w.out[1], gate=gate, residual=x_in, variant=gv)
+        self._linear(w.out, cat, qc, out=x_out, quantize=True, gate=gate, residual=x_in)
 
     # ---------------------------------------------------------------------------------------------------------
     # CoMoE pre-stage (reference preprocess_moe_forward :1028-1068, moe_forward :969-1026, MOELayer.forward,

@@ -10,13 +10,14 @@ from typing import Optional, Sequence
 import torch
 
 from . import _lib
-from ._lib import UG_ACT_GELU_TANH, UG_ACT_NONE, AttnArgs, GemmArgs, QkvScatterArgs, UgError, check
+from ._lib import UG_ACT_GELU_TANH, UG_ACT_NONE, AttnArgs, GemmArgs, GemmFp8Scales, QkvScatterArgs, UgError, check
 
-__all__ = ["gemm", "lora_down", "lora_down_wide", "attention", "attention_peer", "qkv_scatter", "peer_bcast_rows", "peer_barrier", "expand_segment_mask", "ln_modulate", "qk_rmsnorm_rope", "rope_table", "gemv", "GemvPlan", "gemv_grouped", "silu",
+__all__ = ["gemm", "gemm_fp8", "quant_rows_fp8", "ln_modulate_fp8", "lora_down", "lora_down_wide", "attention", "attention_peer", "qkv_scatter", "peer_bcast_rows", "peer_barrier", "expand_segment_mask", "ln_modulate", "qk_rmsnorm_rope", "rope_table", "gemv", "GemvPlan", "gemv_grouped", "silu",
            "timestep_embedding", "add", "copy", "to_bf16", "to_f32", "moe_route", "moe_gather_modulate",
            "moe_combine", "ln_modulate_segs", "ln_modulate_slots", "gated_add_slots", "unpatchify", "euler_step", "euler_step_table", "cfg_combine", "pack_latents", "unpack_latents", "conv3x3", "conv3x3_implicit_ok", "im2col", "groupnorm", "upsample2x", "softmax_rows_", "nhwc_to_nchw", "vae_sample", "launch_count", "reset_launch_count", "UG_ACT_NONE", "UG_ACT_GELU_TANH", "UgError"]
 
 BF16 = torch.bfloat16
+FP8 = torch.float8_e4m3fn
 
 
 def _stream() -> C.c_void_p:
@@ -84,8 +85,37 @@ def gemm(a: torch.Tensor, w: torch.Tensor, out: Optional[torch.Tensor] = None, b
     """out[b,r,:] = residual + alpha * gate[b,:] * act(a[b,r,:] @ w^T + bias (+ switched LoRA update)).
     a: [B,R,K] view, w: [N,K] or [B,N,K]. lora = dict(t=fp32 [B,R,n_blocks*rank] from lora_down, b=bf16 [groups,N,rank]
     (pre-scaled), rank, block_n, seg_bounds, seg_group) applies adapter group seg_group[i] to rows of segment i."""
-    a = _view3(_dev(a, "gemm.a", BF16), "gemm.a")
-    _dev(w, "gemm.w", BF16)
+    g, out = _gemm_args("gemm", BF16, a, w, out, bias, gate, alpha, act, residual, variant, lora, qk_norm, gate_seg_stride,
+                        seg_bounds, a2, w2, colmask)
+    check(_lib.load().ug_gemm_bf16(C.byref(g), _stream()), "ug_gemm_bf16")
+    return out
+
+
+def gemm_fp8(a: torch.Tensor, a_scale: torch.Tensor, w: torch.Tensor, w_scale: torch.Tensor, out: Optional[torch.Tensor] = None,
+             bias: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None, alpha: float = 1.0, act: int = UG_ACT_NONE,
+             residual: Optional[torch.Tensor] = None, variant: int = 0, qk_norm: Optional[dict] = None) -> torch.Tensor:
+    """Row-wise fp8 GEMM: out = residual + alpha * gate * act((a @ w^T) * a_scale[b, r] * w_scale[c] + bias) (or the fused
+    QK-norm epilogue), bf16 out. a: e4m3 [B,R,K] view with a_scale fp32 [B,R] (or [R]); w: e4m3 [N,K] with w_scale fp32 [N]."""
+    g, out = _gemm_args("gemm_fp8", FP8, a, w, out, bias, gate, alpha, act, residual, variant, None, qk_norm)
+    B, R = g.batch, g.rows
+    _dev(a_scale, "gemm_fp8.a_scale", torch.float32), _dev(w_scale, "gemm_fp8.w_scale", torch.float32)
+    s3 = a_scale if a_scale.dim() == 2 else a_scale.unsqueeze(0)
+    if tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
+        raise UgError(f"gemm_fp8: a_scale must be an fp32 [{B}, {R}] view with unit row stride, got {tuple(a_scale.shape)}")
+    if w.dim() != 2 or tuple(w_scale.shape) != (g.n,) or not w_scale.is_contiguous():
+        raise UgError(f"gemm_fp8: w must be [N, K] with a contiguous fp32 w_scale [N] (got w {tuple(w.shape)}, w_scale {tuple(w_scale.shape)})")
+    sc = GemmFp8Scales()
+    sc.a_scale, sc.a_scale_batch_stride = s3.data_ptr(), s3.stride(0)
+    sc.w_scale, sc.w_scale_batch_stride = w_scale.data_ptr(), 0
+    check(_lib.load().ug_gemm_fp8(C.byref(g), C.byref(sc), _stream()), "ug_gemm_fp8")
+    return out
+
+
+def _gemm_args(name, in_dtype, a, w, out, bias, gate, alpha, act, residual, variant, lora, qk_norm, gate_seg_stride=0,
+               seg_bounds=None, a2=None, w2=None, colmask=None):
+    """ug_gemm_args of one launch (shared by gemm and gemm_fp8; the operands a / w are `in_dtype`)."""
+    a = _view3(_dev(a, f"{name}.a", in_dtype), f"{name}.a")
+    _dev(w, f"{name}.w", in_dtype)
     B, R, K = a.shape
     N = w.shape[-2]
     if w.shape[-1] != K:
@@ -164,8 +194,7 @@ def gemm(a: torch.Tensor, w: torch.Tensor, out: Optional[torch.Tensor] = None, b
             if cs.shape[0] < R or not cs.is_contiguous():
                 raise UgError("gemm: qk_norm cos_sin table too short / not contiguous")
             g.qk_cos_sin = cs.data_ptr()
-    check(_lib.load().ug_gemm_bf16(C.byref(g), _stream()), "ug_gemm_bf16")
-    return out
+    return g, out
 
 
 def lora_down(x: torch.Tensor, a_stack: torch.Tensor, seg_bounds: Sequence[int], seg_group: Sequence[int],
@@ -307,6 +336,43 @@ def ln_modulate(x: torch.Tensor, out: torch.Tensor, shift: torch.Tensor, scale: 
                                      shift.data_ptr(), scale.data_ptr(), shift.stride(0), B, R, D, float(eps), _stream()),
           "ug_ln_modulate")
     return out
+
+
+def quant_rows_fp8(x: torch.Tensor, out: Optional[torch.Tensor] = None, scale: Optional[torch.Tensor] = None):
+    """Dynamic row-wise e4m3 quantisation of a bf16 [B, R, K] (or [R, K]) view -> (out e4m3 [B, R, K], scale fp32 [B, R]):
+    scale = amax / 448 (1 for an all-zero row), out = satfinite_e4m3(x * 448 / amax). out / scale may be views (unit inner
+    strides) into larger buffers; they are allocated contiguous otherwise."""
+    x3 = _view3(_dev(x, "quant_rows_fp8.x", BF16), "quant_rows_fp8.x")
+    B, R, K = x3.shape
+    if out is None:
+        out = torch.empty(x.shape, device=x.device, dtype=FP8)
+    if scale is None:
+        scale = torch.empty(x.shape[:-1], device=x.device, dtype=torch.float32)
+    q3 = _view3(_dev(out, "quant_rows_fp8.out", FP8), "quant_rows_fp8.out")
+    s3 = _dev(scale, "quant_rows_fp8.scale", torch.float32)
+    s3 = s3 if s3.dim() == 2 else s3.unsqueeze(0)
+    if tuple(q3.shape) != (B, R, K) or tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
+        raise UgError(f"quant_rows_fp8: out {tuple(out.shape)} / scale {tuple(scale.shape)} do not match x {tuple(x.shape)}")
+    check(_lib.load().ug_quant_rows_fp8(x3.data_ptr(), x3.stride(1), x3.stride(0), q3.data_ptr(), q3.stride(1), q3.stride(0),
+                                        s3.data_ptr(), s3.stride(0), B, R, K, _stream()), "ug_quant_rows_fp8")
+    return out, scale
+
+
+def ln_modulate_fp8(x: torch.Tensor, out: torch.Tensor, out_scale: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor,
+                    eps: float = 1e-6):
+    """quant_rows_fp8(ln_modulate(x, shift, scale)) in one pass, bit for bit: out e4m3 [B, R, D] view, out_scale fp32 [B, R]."""
+    x3, q3 = _view3(_dev(x, "ln_fp8.x", BF16), "ln_fp8.x"), _view3(_dev(out, "ln_fp8.out", FP8), "ln_fp8.out")
+    _dev(shift, "ln_fp8.shift", torch.float32), _dev(scale, "ln_fp8.scale", torch.float32), _dev(out_scale, "ln_fp8.out_scale", torch.float32)
+    B, R, D = x3.shape
+    s3 = out_scale if out_scale.dim() == 2 else out_scale.unsqueeze(0)
+    if tuple(q3.shape) != (B, R, D) or tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
+        raise UgError(f"ln_modulate_fp8: out {tuple(out.shape)} / out_scale {tuple(out_scale.shape)} do not match x {tuple(x.shape)}")
+    if shift.stride(0) != scale.stride(0) and B > 1:
+        raise UgError("ln_modulate_fp8: shift and scale need the same batch stride")
+    check(_lib.load().ug_ln_modulate_fp8(x3.data_ptr(), x3.stride(1), x3.stride(0), q3.data_ptr(), q3.stride(1), q3.stride(0),
+                                         s3.data_ptr(), s3.stride(0), shift.data_ptr(), scale.data_ptr(), shift.stride(0), B, R, D,
+                                         float(eps), _stream()), "ug_ln_modulate_fp8")
+    return out, out_scale
 
 
 def ln_modulate_segs(x: torch.Tensor, out: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor, seg_bounds: Sequence[int],

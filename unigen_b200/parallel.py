@@ -232,6 +232,8 @@ class SequenceParallelUniGenFlux(UniGenFlux):
             return super()._run_staged((key, "local"), staged, *args)
         if self.use_consis_module and self.use_shared_expert:
             raise ops.UgError("use_consis_module is not sharded: run with sp_enabled=False (the pre-stage is a small part of the step)")
+        if self.linear_dtype != torch.bfloat16:
+            raise ops.UgError("fp8-quantised block linears (quantize_fp8) are not sharded: run with sp_enabled=False or a bf16 model")
         if self.exchange != "peer":  # NCCL collectives stay out of graph capture: the staged-exchange baseline runs eagerly
             return self._forward_impl(*args, **staged)
         if self._pool is not None:
