@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define UG_ABI_VERSION 10
+#define UG_ABI_VERSION 11
 
 typedef enum {
   UG_OK = 0,
@@ -149,6 +149,19 @@ typedef struct ug_gemm_fp8_scales {
 } ug_gemm_fp8_scales;
 int ug_gemm_fp8(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream);
 
+/* ug_gemm_fp8 plus the two switched-LoRA features of the P-variant (`UniCombineFlux.quantize_fp8()`), on their own kernel
+ * instances (the ones behind ug_gemm_fp8 are unchanged):
+ *   - a bf16 second operand pair (a2 / w2 / k2, ug_gemm_args): its K blocks run as kind::f16 MMAs into the SAME fp32 accumulator
+ *     as the e4m3 blocks, so the dequantisation multiplies both:  out = a_s[r] w_s[c] (sum_k q[r,k] Wq[c,k] + sum_j A2[r,j] W2[c,j]).
+ *     For the LoRA update x A^T B^T pass the pre-divided operands A2 = (x / a_s) A^T and W2 = B / w_s[c] (the scaling is rank-1
+ *     separable, so this is exact up to the bf16 rounding of A2 / W2);
+ *   - colmask_block with its segment table (the masked grouped down-projection).
+ * a_scale == NULL reads as unit row scales: with (q, a_s) = the quantised operand of x and W = the quantised stacked lora_A
+ * (per-row scales aw_s) this gives A2 = q @ Aq^T * aw_s = (x / a_s) A^T directly. Tile variants, the auto picker and every
+ * epilogue (direct, staged, fused QK-norm + RoPE, gate_seg_stride, bias, GELU, residual) are those of ug_gemm_fp8. Rejected:
+ * lora_t, k % 16 != 0, a NULL w_scale. (The implicit-GEMM convolution is bf16-only: ug_conv3x3_bf16 has no fp8 form.) */
+int ug_gemm_fp8_lora(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream);
+
 /* Dynamic row-wise quantisation of bf16 [batch, rows, k] (strided) to e4m3 [batch, rows, k] plus one fp32 scale per row:
  *   amax = max |x|;  amax == 0: scale = 1, q = 0;  else inv = 448 / amax, scale = amax / 448 (IEEE divisions),
  *   q = cvt.rn.satfinite.e4m3(x * inv)        == torch (x.float() * inv).clamp(-448, 448).to(torch.float8_e4m3fn)
@@ -235,6 +248,13 @@ int ug_ln_modulate_segs(const void* x, int64_t x_row_stride, int64_t x_batch_str
                         int64_t o_batch_stride, const float* shift, const float* scale, int64_t mod_batch_stride,
                         int64_t mod_seg_stride, int32_t nseg, const int32_t* seg_bounds_host, int32_t batch, int32_t rows,
                         int32_t d, float eps, void* stream);
+
+/* ug_ln_modulate_segs with the e4m3 output of ug_ln_modulate_fp8: (q, q_scale) equal ug_quant_rows_fp8(ug_ln_modulate_segs(x))
+ * bit for bit. The shared operand of a quantised P-variant block's text, image / condition and LoRA down-projection GEMMs. */
+int ug_ln_modulate_segs_fp8(const void* x, int64_t x_row_stride, int64_t x_batch_stride, void* q, int64_t q_row_stride,
+                            int64_t q_batch_stride, float* q_scale, int64_t q_scale_batch_stride, const float* shift,
+                            const float* scale, int64_t mod_batch_stride, int64_t mod_seg_stride, int32_t nseg,
+                            const int32_t* seg_bounds_host, int32_t batch, int32_t rows, int32_t d, float eps, void* stream);
 
 /* Per-token AdaLN on capacity-slot buffers — the SD3.5 transformer-block experts run `SD3SingleTransformerBlock` on the
  * dispatched (1, C, D) chunks with a PER-TOKEN (1, C, D) temb (src/UniGenUtils.py:354-363,386-414 with a 3-D `emb`;

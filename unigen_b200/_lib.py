@@ -12,7 +12,7 @@ UG_ACT_NONE = 0
 UG_ACT_GELU_TANH = 1
 UG_MAX_SEGMENTS = 8
 UG_GROUPNORM_MAX_CHUNKS = 1024
-UG_ABI_VERSION = 10  # include/unigen_b200.h; checked against ug_abi_version() of the loaded library
+UG_ABI_VERSION = 11  # include/unigen_b200.h; checked against ug_abi_version() of the loaded library
 
 
 class UgError(RuntimeError):
@@ -123,6 +123,7 @@ SIGNATURES = {
     "ug_reset_launch_count": (None, []),
     "ug_gemm_bf16": (C.c_int, [C.POINTER(GemmArgs), _VP]),
     "ug_gemm_fp8": (C.c_int, [C.POINTER(GemmArgs), C.POINTER(GemmFp8Scales), _VP]),
+    "ug_gemm_fp8_lora": (C.c_int, [C.POINTER(GemmArgs), C.POINTER(GemmFp8Scales), _VP]),
     "ug_quant_rows_fp8": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _I64, _I32, _I32, _I32, _VP]),
     "ug_ln_modulate_fp8": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _I64, _VP, _VP, _I64, _I32, _I32, _I32, _F32, _VP]),
     "ug_lora_down": (C.c_int, [_VP, _I64, _I64, _VP, _VP, _I64, _I64, _I32, _I32, _I32, _I32, _I32,
@@ -134,6 +135,8 @@ SIGNATURES = {
     "ug_ln_modulate": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _VP, _I64, _I32, _I32, _I32, _F32, _VP]),
     "ug_ln_modulate_segs": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _VP, _I64, _I64, _I32, C.POINTER(C.c_int32), _I32, _I32,
                                       _I32, _F32, _VP]),
+    "ug_ln_modulate_segs_fp8": (C.c_int, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _I64, _VP, _VP, _I64, _I64, _I32, C.POINTER(C.c_int32),
+                                          _I32, _I32, _I32, _F32, _VP]),
     "ug_ln_modulate_slots": (C.c_int, [_VP, _I64, _VP, _I64, _VP, _VP, _I64, _I64, _VP, _I32, _I32, _I32, _I32, _I32, _F32, _VP]),
     "ug_gated_add_slots": (C.c_int, [_VP, _I64, _VP, _I64, _VP, _I64, _I64, _VP, _I32, _I32, _I32, _I32, _I32, _VP]),
     "ug_qk_rmsnorm_rope": (C.c_int, [_VP, _I64, _I64, _I32, _I32, _I32, _I32, _VP, _I32, _F32, _VP, _VP]),

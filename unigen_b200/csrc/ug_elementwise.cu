@@ -1064,6 +1064,24 @@ extern "C" int ug_ln_modulate_segs(const void* x, int64_t x_rs, int64_t x_bs, vo
                             "ln_modulate_segs", segs, mod_seg_stride);
 }
 
+extern "C" int ug_ln_modulate_segs_fp8(const void* x, int64_t x_rs, int64_t x_bs, void* q, int64_t q_rs, int64_t q_bs, float* q_scale,
+                                       int64_t q_scale_bs, const float* shift, const float* scale, int64_t mod_bs,
+                                       int64_t mod_seg_stride, int32_t nseg, const int32_t* seg_bounds, int32_t batch, int32_t rows,
+                                       int32_t d, float eps, void* stream) {
+  UG_CHECK_ARG(seg_bounds && nseg >= 1 && nseg <= UG_MAX_SEGMENTS && mod_seg_stride % 4 == 0, "ln_modulate_segs_fp8: bad segment table");
+  UG_CHECK_ARG(q && q_scale, "ln_modulate_segs_fp8: null output pointer");
+  UG_CHECK_ARG((reinterpret_cast<uintptr_t>(q) & 7) == 0 && q_rs % 8 == 0 && q_bs % 8 == 0 && (reinterpret_cast<uintptr_t>(q_scale) & 3) == 0,
+               "ln_modulate_segs_fp8: e4m3 rows must be 8-byte aligned");
+  UG_CHECK_ARG(batch == 1 || q_bs >= (int64_t)rows * q_rs, "ln_modulate_segs_fp8: overlapping output batches");
+  ug::RowSegs segs;
+  segs.nseg = nseg;
+  for (int i = 0; i <= UG_MAX_SEGMENTS; ++i) segs.bounds[i] = i <= nseg ? seg_bounds[i] : rows;
+  // `out` is never written in the fp8 form: the input pointer stands in for it in the shared argument checks
+  return launch_ln_modulate(x, x_rs, x_bs, const_cast<void*>(x), x_rs, x_bs, shift, scale, mod_bs, batch, rows, d, eps, nullptr, 1, 1,
+                            0, 0, stream, "ln_modulate_segs_fp8", segs, mod_seg_stride,
+                            ug::Fp8Out{static_cast<uint8_t*>(q), q_rs, q_bs, q_scale, q_scale_bs});
+}
+
 extern "C" int ug_ln_modulate_slots(const void* x, int64_t x_rs, void* out, int64_t o_rs, const float* shift, const float* scale,
                                     int64_t mod_expert_stride, int64_t mod_index_stride, const int32_t* slot_token,
                                     int32_t experts, int32_t capacity, int32_t tokens_per_batch, int32_t empty_index, int32_t d,

@@ -2,6 +2,8 @@
 // double-buffered) -> fused epilogue from TMEM (bias / GELU-tanh / gate * alpha / residual) -> HBM.
 // kFp8 instances read e4m3 operands (kind::f8f6f4, one 128-byte swizzle row = 128 elements, so stage bytes, TMA boxes and
 // smem descriptors keep their sizes) and dequantise the accumulator with per-row / per-channel scales before the epilogue.
+// kExt16 (fp8 only): the second operand pair (K extension) stays bf16 — its K blocks are 64 bf16 = the same 128-byte swizzle
+// row, issued as kind::f16 MMAs into the accumulator the kind::f8f6f4 MMAs of the first pair started.
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM owner), warps 2..9 = epilogue
 // (warp w reads TMEM lanes 32*(w%4)..+31, the hardware lane-quarter rule of tcgen05.ld; the two warps that share a lane
@@ -365,7 +367,7 @@ __device__ __forceinline__ void tile_coords(const GemmParams& p, int tile, int m
   nt = in_band / size;
 }
 
-template <int kCta, int BN, int kStages, bool kTmaEpi, bool kFp8>
+template <int kCta, int BN, int kStages, bool kTmaEpi, bool kFp8, bool kExt16>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w,
                  const __grid_constant__ CUtensorMap tma_a2, const __grid_constant__ CUtensorMap tma_w2,
@@ -457,7 +459,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             const bool second = kb >= p.k1_blocks;
             const CUtensorMap* ma = second ? &tma_a2 : &tma_a;
             const CUtensorMap* mw = second ? &tma_w2 : &tma_w;
-            const int kc = (second ? kb - p.k1_blocks : kb) * Cfg::BK;
+            const int kc = second ? (kb - p.k1_blocks) * (kExt16 ? 64 : Cfg::BK) : kb * Cfg::BK;
             if constexpr (kCta == 1) {
               mbar_arrive_expect_tx(&full[stage], Cfg::STAGE_BYTES);
               tma_load_3d(sa, ma, &full[stage], kc, row0, b);
@@ -495,10 +497,17 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           if (elect_one_sync()) {
             const uint64_t a_desc = make_sdesc_sw128(smem_u32(smem_a + stage * Cfg::A_BYTES), 16, 1024);
             const uint64_t b_desc = make_sdesc_sw128(smem_u32(smem_b + stage * Cfg::B_BYTES), 16, 1024);
+            if (kExt16 && kb >= p.k1_blocks) {
+              // bf16 K-extension block (kb >= 1: always accumulates onto the fp8 partial sums)
+              constexpr uint32_t idesc16 = make_idesc_bf16(Cfg::BM * kCta, BN, false, false);
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              // +32 bytes per K step (16 bf16 / 32 e4m3) inside the 128-byte swizzle row (start-address field is in 16 B units)
-              umma_ss<kCta, kFp8>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
+              for (int k = 0; k < 4; ++k) umma_ss<kCta, false>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc16, 1u);
+            } else {
+#pragma unroll
+              for (int k = 0; k < 4; ++k) {
+                // +32 bytes per K step (16 bf16 / 32 e4m3) inside the 128-byte swizzle row (start-address field is in 16 B units)
+                umma_ss<kCta, kFp8>(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
+              }
             }
             if constexpr (kCta == 1) {
               umma_commit(&empty[stage]);
@@ -536,7 +545,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
       const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + as * BN;
       const int lora_g = (p.lora_t || p.colmask_block) ? lora_group_of(p, r) : -1;
       // fp8: this row's activation scale (rows past the matrix edge are computed, never stored: read a valid entry)
-      const float a_s = kFp8 ? __ldg(p.a_scale + (long long)b * p.a_scale_bs + min(r, p.rows - 1)) : 1.f;
+      // (kExt16: a NULL a_scale means unit scales — the masked down-projection of the LoRA operand A2)
+      const float a_s = !kFp8 || (kExt16 && !p.a_scale) ? 1.f : __ldg(p.a_scale + (long long)b * p.a_scale_bs + min(r, p.rows - 1));
       (void)a_s;
       // gate vector of this row: per sample, and per row segment when gate_seg_stride is set (once per tile, not per chunk)
       const float* gate_row = p.gate ? p.gate + (long long)b * p.gate_bs + (p.gate_seg_stride ? seg_index_of(p, r) * p.gate_seg_stride : 0)
@@ -706,17 +716,19 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   }
 }
 
-template <int kCta, int BN, int kStages, bool kTmaEpi = false, bool kFp8 = false>
+template <int kCta, int BN, int kStages, bool kTmaEpi = false, bool kFp8 = false, bool kExt16 = false>
 static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDesc* conv = nullptr,
                        const ug_gemm_fp8_scales* scales = nullptr) {
   using Cfg = GemmCfg<kCta, BN, kStages, kTmaEpi, kFp8>;
   constexpr uint64_t E = Cfg::ESIZE;
+  constexpr int BK2 = kExt16 ? 64 : Cfg::BK;  // K block of the second operand pair (always bf16: 64 = one swizzle row)
+  static_assert(!kExt16 || kFp8, "kExt16 is the bf16 K extension of an fp8 GEMM");
   // A / W operand maps: bf16, or one e4m3 per byte (UINT8) for the fp8 instances
   auto encode_op = [](CUtensorMap* m, const void* base, int rank, const uint64_t* dims, const uint64_t* strides, const uint32_t* box) {
     return kFp8 ? encode_tmap(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, base, rank, dims, strides, box)
                 : encode_tmap_bf16(m, base, rank, dims, strides, box);
   };
-  auto kern = gemm_bf16_kernel<kCta, BN, kStages, kTmaEpi, kFp8>;
+  auto kern = gemm_bf16_kernel<kCta, BN, kStages, kTmaEpi, kFp8, kExt16>;
   static bool attr_done[64] = {false};
   if (int st = ensure_dynamic_smem(kern, Cfg::SMEM_BYTES, attr_done, "gemm"); st != UG_OK) return st;
   CUtensorMap tma_a, tma_w;
@@ -753,18 +765,18 @@ static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDes
       uint64_t dims[3] = {(uint64_t)a.k2, (uint64_t)a.rows, (uint64_t)a.batch};
       uint64_t bs = a.batch > 1 ? (uint64_t)a.a2_batch_stride : (uint64_t)a.rows * a.a2_row_stride;
       uint64_t strides[2] = {(uint64_t)a.a2_row_stride * 2, bs * 2};
-      uint32_t box[3] = {(uint32_t)Cfg::BK, (uint32_t)Cfg::BM, 1};
+      uint32_t box[3] = {(uint32_t)BK2, (uint32_t)Cfg::BM, 1};
       int st = encode_tmap_bf16(&tma_a2, a.a2, 3, dims, strides, box);
       if (st != UG_OK) return st;
     }
     {
       uint64_t dims[3] = {(uint64_t)a.k2, (uint64_t)a.n, 1};
       uint64_t strides[2] = {(uint64_t)a.w2_row_stride * 2, (uint64_t)a.n * a.w2_row_stride * 2};
-      uint32_t box[3] = {(uint32_t)Cfg::BK, (uint32_t)Cfg::BN_LOAD, 1};
+      uint32_t box[3] = {(uint32_t)BK2, (uint32_t)Cfg::BN_LOAD, 1};
       int st = encode_tmap_bf16(&tma_w2, a.w2, 3, dims, strides, box);
       if (st != UG_OK) return st;
     }
-    k2_blocks = (a.k2 + Cfg::BK - 1) / Cfg::BK;
+    k2_blocks = (a.k2 + BK2 - 1) / BK2;
   }
   CUtensorMap tma_c = tma_a, tma_r = tma_a;
   if constexpr (kTmaEpi) {
@@ -791,12 +803,13 @@ static int launch_gemm(const ug_gemm_args& a, cudaStream_t stream, const ConvDes
   p.n_tiles = (a.n + BN - 1) / BN;
   {
     // A bytes one sweep over all m-tiles touches; above ~40 MB it no longer survives in the 126 MB L2 between n-waves
-    const long long a_bytes = (long long)a.batch * a.rows * (a.k + (a.a2 ? a.k2 : 0)) * Cfg::ESIZE;
+    const long long row_bytes = (long long)a.k * Cfg::ESIZE + (a.a2 ? 2LL * a.k2 : 0LL);  // the second pair is bf16
+    const long long a_bytes = (long long)a.batch * a.rows * row_bytes;
     const int mb_all = p.m_tiles * a.batch;
     p.group_m = mb_all;
     if (a_bytes > (40LL << 20) && !(a.w_batch_stride != 0 && a.batch > 1)) {
       // band of A row-tiles worth ~24 MB: it stays in L2 while the band sweeps every n-tile, so A is read from HBM once
-      const long long tile_bytes = (long long)Cfg::BM * kCta * (a.k + (a.a2 ? a.k2 : 0)) * Cfg::ESIZE;
+      const long long tile_bytes = (long long)Cfg::BM * kCta * row_bytes;
       long long gm = (24LL << 20) / tile_bytes;
       gm = gm < 2 ? 2 : (gm > 16 ? 16 : gm);
       p.group_m = gm < mb_all ? (int)gm : mb_all;
@@ -877,23 +890,24 @@ static int pick_tile_variant(int batch, int rows, int n) {
   return variant;
 }
 
-template <bool kFp8>
+template <bool kFp8, bool kExt16 = false>
 static int launch_variant(int variant, const ug_gemm_args& a, cudaStream_t s, const ug_gemm_fp8_scales* scales) {
   switch (variant) {
-    case 1: return launch_gemm<1, 256, 4, false, kFp8>(a, s, nullptr, scales);
-    case 2: return launch_gemm<2, 256, 6, false, kFp8>(a, s, nullptr, scales);
-    case 3: return launch_gemm<1, 128, 6, false, kFp8>(a, s, nullptr, scales);
-    case 4: return launch_gemm<2, 256, 5, true, kFp8>(a, s, nullptr, scales);
-    case 5: return launch_gemm<1, 256, 3, true, kFp8>(a, s, nullptr, scales);
-    case 6: return launch_gemm<1, 128, 6, true, kFp8>(a, s, nullptr, scales);
+    case 1: return launch_gemm<1, 256, 4, false, kFp8, kExt16>(a, s, nullptr, scales);
+    case 2: return launch_gemm<2, 256, 6, false, kFp8, kExt16>(a, s, nullptr, scales);
+    case 3: return launch_gemm<1, 128, 6, false, kFp8, kExt16>(a, s, nullptr, scales);
+    case 4: return launch_gemm<2, 256, 5, true, kFp8, kExt16>(a, s, nullptr, scales);
+    case 5: return launch_gemm<1, 256, 3, true, kFp8, kExt16>(a, s, nullptr, scales);
+    case 6: return launch_gemm<1, 128, 6, true, kFp8, kExt16>(a, s, nullptr, scales);
     default:
       set_error("gemm: unknown variant %d", a.variant);
       return UG_ERR_INVALID;
   }
 }
 
-// ug_gemm_bf16 (scales == NULL) and ug_gemm_fp8: argument checks, tile / epilogue choice, launch
-static int gemm_entry(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream) {
+// ug_gemm_bf16 (scales == NULL), ug_gemm_fp8 and ug_gemm_fp8_lora (lora: bf16 K extension + column mask allowed, NULL
+// a_scale = unit row scales): argument checks, tile / epilogue choice, launch
+static int gemm_entry(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream, bool lora = false) {
   const bool fp8 = scales != nullptr;
   UG_CHECK_ARG(args != nullptr, "gemm: null args");
   const ug_gemm_args& a = *args;
@@ -907,9 +921,15 @@ static int gemm_entry(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales
     UG_CHECK_ARG(a.a_row_stride % 16 == 0 && a.w_row_stride % 16 == 0 && (a.batch == 1 || a.a_batch_stride % 16 == 0) &&
                      a.w_batch_stride % 16 == 0,
                  "gemm_fp8: e4m3 row / batch strides must be multiples of 16 elements (16 bytes)");
-    UG_CHECK_ARG(!a.lora_t && !a.colmask_block && !a.a2 && !a.w2,
-                 "gemm_fp8: lora_t, colmask_block and the second operand pair (a2 / w2) are bf16-only");
-    UG_CHECK_ARG(scales->a_scale && scales->w_scale, "gemm_fp8: null a_scale / w_scale");
+    if (lora) {
+      UG_CHECK_ARG(!a.lora_t, "gemm_fp8_lora: lora_t (the update in the epilogue) is bf16-only: pass it as the K extension a2 / w2");
+      UG_CHECK_ARG(!a.a2 == !a.w2, "gemm_fp8_lora: a2 and w2 go together");
+      UG_CHECK_ARG(scales->w_scale, "gemm_fp8_lora: null w_scale");
+    } else {
+      UG_CHECK_ARG(!a.lora_t && !a.colmask_block && !a.a2 && !a.w2,
+                   "gemm_fp8: lora_t, colmask_block and the second operand pair (a2 / w2) are bf16-only");
+      UG_CHECK_ARG(scales->a_scale && scales->w_scale, "gemm_fp8: null a_scale / w_scale");
+    }
     UG_CHECK_ARG((reinterpret_cast<uintptr_t>(scales->a_scale) & 3) == 0 && (reinterpret_cast<uintptr_t>(scales->w_scale) & 15) == 0 &&
                      scales->w_scale_batch_stride % 4 == 0,
                  "gemm_fp8: w_scale must be 16-byte aligned (batch stride a multiple of 4), a_scale 4-byte aligned");
@@ -988,6 +1008,7 @@ static int gemm_entry(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales
                  "gemm: the staged fused QK-norm epilogue needs a 256-column tile (variants 4 / 5) and qk_d a multiple of 128");
     UG_CHECK_ARG(!a.residual || a.res_batch_stride % 8 == 0 || a.batch == 1, "gemm: residual batch stride must be a multiple of 8");
   }
+  if (lora) return launch_variant<true, true>(variant, a, s, scales);
   return fp8 ? launch_variant<true>(variant, a, s, scales) : launch_variant<false>(variant, a, s, nullptr);
 }
 
@@ -1003,6 +1024,18 @@ extern "C" int ug_gemm_fp8(const ug_gemm_args* args, const ug_gemm_fp8_scales* s
     return UG_ERR_INVALID;
   }
   return ug::gemm_entry(args, scales, stream);
+}
+
+// The fp8 GEMM with the two switched-LoRA features of the P-variant: a bf16 second operand pair (K extension, kind::f16 MMAs
+// into the fp8 accumulator: its operands arrive pre-divided by the scales the epilogue multiplies with) and the column mask of
+// the grouped down-projection. A NULL a_scale reads as unit row scales. A separate set of kernel instances (kExt16), so the
+// instances behind ug_gemm_fp8 keep their code. An opt-in path of `UniCombineFlux.quantize_fp8()`.
+extern "C" int ug_gemm_fp8_lora(const ug_gemm_args* args, const ug_gemm_fp8_scales* scales, void* stream) {
+  if (scales == nullptr) {
+    ug::set_error("gemm_fp8_lora: null scales");
+    return UG_ERR_INVALID;
+  }
+  return ug::gemm_entry(args, scales, stream, true);
 }
 
 // 3x3 convolution, stride 1, zero padding 1, over NHWC bf16 images as an implicit GEMM on the tcgen05 path above: no im2col

@@ -76,7 +76,7 @@ class _Weights:
 
 
 class _DoubleBlockW:
-    # linears `UniGenFlux.quantize_fp8()` converts; once it has, `fp8` is True and each of them is (W e4m3 [N, K], bias bf16 [N],
+    # linears `UniGenFlux.quantize_fp8()` / `UniCombineFlux.quantize_fp8()` convert; once they have, `fp8` is True and each of them is (W e4m3 [N, K], bias bf16 [N],
     # w_scale fp32 [N]) instead of (W bf16, bias)
     FP8_LINEARS = ("qkv", "add_qkv", "to_out", "to_add_out", "ff1", "ff2", "ffc1", "ffc2")
     fp8 = False
@@ -109,6 +109,21 @@ class _SingleBlockW:
         self.out = ws.linear(p + ".proj_out", D, 5 * D)
         self.rms = ws.alloc(2, dh)
         ws.views[p + ".attn.norm_q.weight"], ws.views[p + ".attn.norm_k.weight"] = self.rms[0], self.rms[1]
+
+
+def quantize_block_linears(ws: _Weights, blocks) -> None:
+    """Every linear named in a block's FP8_LINEARS becomes (W e4m3 [N, K], bias bf16 [N], w_scale fp32 [N]), one scale per output
+    channel; the bf16 weight is released and its state-dict views are dropped (the bias stays). Marks the blocks `fp8`."""
+    views = ws.views
+    for w in blocks:
+        for name in w.FP8_LINEARS:
+            W, bias = getattr(w, name)
+            q, w_scale = ops.quant_rows_fp8(W)  # a row of W is an output channel
+            ptr = W.untyped_storage().data_ptr()
+            for k in [k for k, v in views.items() if k.endswith(".weight") and v.untyped_storage().data_ptr() == ptr]:
+                del views[k]
+            setattr(w, name, (q, bias, w_scale))
+        w.fp8 = True
 
 
 class _TimeTextW:
@@ -397,16 +412,7 @@ class UniGenFlux(_DenoiserBase):
             raise ops.UgError("call init_condition_block(condition_nums=..., control_params=...) before quantize_fp8()")
         if self.linear_dtype == FP8:
             return self
-        views = self._ws.views
-        for w in self.double + self.ctrl_double + self.single + self.ctrl_single:
-            for name in w.FP8_LINEARS:
-                W, bias = getattr(w, name)
-                q, w_scale = ops.quant_rows_fp8(W)  # a row of W is an output channel
-                ptr = W.untyped_storage().data_ptr()
-                for k in [k for k, v in views.items() if k.endswith(".weight") and v.untyped_storage().data_ptr() == ptr]:
-                    del views[k]
-                setattr(w, name, (q, bias, w_scale))
-            w.fp8 = True
+        quantize_block_linears(self._ws, self.double + self.ctrl_double + self.single + self.ctrl_single)
         self.linear_dtype = FP8
         # workspaces (and the graphs captured over them, the pipeline's whole-loop graphs included) hold bf16 operands only
         from .pipeline import _GRAPHS_ATTR

@@ -14,7 +14,7 @@ from ._lib import UG_ACT_GELU_TANH, UG_ACT_NONE, AttnArgs, GemmArgs, GemmFp8Scal
 
 __all__ = ["gemm", "gemm_fp8", "quant_rows_fp8", "ln_modulate_fp8", "lora_down", "lora_down_wide", "attention", "attention_peer", "qkv_scatter", "peer_bcast_rows", "peer_barrier", "expand_segment_mask", "ln_modulate", "qk_rmsnorm_rope", "rope_table", "gemv", "GemvPlan", "gemv_grouped", "silu",
            "timestep_embedding", "add", "copy", "to_bf16", "to_f32", "moe_route", "moe_gather_modulate",
-           "moe_combine", "ln_modulate_segs", "ln_modulate_slots", "gated_add_slots", "unpatchify", "euler_step", "euler_step_table", "cfg_combine", "pack_latents", "unpack_latents", "conv3x3", "conv3x3_implicit_ok", "im2col", "groupnorm", "upsample2x", "softmax_rows_", "nhwc_to_nchw", "vae_sample", "launch_count", "reset_launch_count", "UG_ACT_NONE", "UG_ACT_GELU_TANH", "UgError"]
+           "moe_combine", "ln_modulate_segs", "ln_modulate_segs_fp8", "ln_modulate_slots", "gated_add_slots", "unpatchify", "euler_step", "euler_step_table", "cfg_combine", "pack_latents", "unpack_latents", "conv3x3", "conv3x3_implicit_ok", "im2col", "groupnorm", "upsample2x", "softmax_rows_", "nhwc_to_nchw", "vae_sample", "launch_count", "reset_launch_count", "UG_ACT_NONE", "UG_ACT_GELU_TANH", "UgError"]
 
 BF16 = torch.bfloat16
 FP8 = torch.float8_e4m3fn
@@ -91,23 +91,37 @@ def gemm(a: torch.Tensor, w: torch.Tensor, out: Optional[torch.Tensor] = None, b
     return out
 
 
-def gemm_fp8(a: torch.Tensor, a_scale: torch.Tensor, w: torch.Tensor, w_scale: torch.Tensor, out: Optional[torch.Tensor] = None,
+def gemm_fp8(a: torch.Tensor, a_scale: Optional[torch.Tensor], w: torch.Tensor, w_scale: torch.Tensor, out: Optional[torch.Tensor] = None,
              bias: Optional[torch.Tensor] = None, gate: Optional[torch.Tensor] = None, alpha: float = 1.0, act: int = UG_ACT_NONE,
-             residual: Optional[torch.Tensor] = None, variant: int = 0, qk_norm: Optional[dict] = None) -> torch.Tensor:
+             residual: Optional[torch.Tensor] = None, variant: int = 0, qk_norm: Optional[dict] = None, gate_seg_stride: int = 0,
+             seg_bounds: Optional[Sequence[int]] = None, a2: Optional[torch.Tensor] = None, w2: Optional[torch.Tensor] = None,
+             colmask: Optional[dict] = None) -> torch.Tensor:
     """Row-wise fp8 GEMM: out = residual + alpha * gate * act((a @ w^T) * a_scale[b, r] * w_scale[c] + bias) (or the fused
-    QK-norm epilogue), bf16 out. a: e4m3 [B,R,K] view with a_scale fp32 [B,R] (or [R]); w: e4m3 [N,K] with w_scale fp32 [N]."""
-    g, out = _gemm_args("gemm_fp8", FP8, a, w, out, bias, gate, alpha, act, residual, variant, None, qk_norm)
+    QK-norm epilogue), bf16 out. a: e4m3 [B,R,K] view with a_scale fp32 [B,R] (or [R]); w: e4m3 [N,K] with w_scale fp32 [N].
+    With a bf16 K extension a2 [B,R,K2] / w2 [N,K2] or a column mask (as in `gemm`) it runs ug_gemm_fp8_lora: the accumulator
+    a @ w^T + a2 @ w2^T is dequantised as a whole, so a2 / w2 carry the low-rank update pre-divided by a_scale / w_scale; there
+    a_scale=None means unit row scales (the masked down-projection of a quantised operand)."""
+    g, out = _gemm_args("gemm_fp8", FP8, a, w, out, bias, gate, alpha, act, residual, variant, None, qk_norm, gate_seg_stride,
+                        seg_bounds, a2, w2, colmask)
+    lora = a2 is not None or colmask is not None
     B, R = g.batch, g.rows
-    _dev(a_scale, "gemm_fp8.a_scale", torch.float32), _dev(w_scale, "gemm_fp8.w_scale", torch.float32)
-    s3 = a_scale if a_scale.dim() == 2 else a_scale.unsqueeze(0)
-    if tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
-        raise UgError(f"gemm_fp8: a_scale must be an fp32 [{B}, {R}] view with unit row stride, got {tuple(a_scale.shape)}")
+    _dev(w_scale, "gemm_fp8.w_scale", torch.float32)
+    sc = GemmFp8Scales()
+    if a_scale is None and not lora:
+        raise UgError("gemm_fp8: a_scale is required (None = unit row scales only with a2 / w2 or colmask)")
+    if a_scale is not None:
+        _dev(a_scale, "gemm_fp8.a_scale", torch.float32)
+        s3 = a_scale if a_scale.dim() == 2 else a_scale.unsqueeze(0)
+        if tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
+            raise UgError(f"gemm_fp8: a_scale must be an fp32 [{B}, {R}] view with unit row stride, got {tuple(a_scale.shape)}")
+        sc.a_scale, sc.a_scale_batch_stride = s3.data_ptr(), s3.stride(0)
     if w.dim() != 2 or tuple(w_scale.shape) != (g.n,) or not w_scale.is_contiguous():
         raise UgError(f"gemm_fp8: w must be [N, K] with a contiguous fp32 w_scale [N] (got w {tuple(w.shape)}, w_scale {tuple(w_scale.shape)})")
-    sc = GemmFp8Scales()
-    sc.a_scale, sc.a_scale_batch_stride = s3.data_ptr(), s3.stride(0)
     sc.w_scale, sc.w_scale_batch_stride = w_scale.data_ptr(), 0
-    check(_lib.load().ug_gemm_fp8(C.byref(g), C.byref(sc), _stream()), "ug_gemm_fp8")
+    if lora:
+        check(_lib.load().ug_gemm_fp8_lora(C.byref(g), C.byref(sc), _stream()), "ug_gemm_fp8_lora")
+    else:
+        check(_lib.load().ug_gemm_fp8(C.byref(g), C.byref(sc), _stream()), "ug_gemm_fp8")
     return out
 
 
@@ -387,6 +401,24 @@ def ln_modulate_segs(x: torch.Tensor, out: torch.Tensor, shift: torch.Tensor, sc
                                           shift.data_ptr(), scale.data_ptr(), shift.stride(0), int(mod_seg_stride), n, sb, B, R, D,
                                           float(eps), _stream()), "ug_ln_modulate_segs")
     return out
+
+
+def ln_modulate_segs_fp8(x: torch.Tensor, out: torch.Tensor, out_scale: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor,
+                         seg_bounds: Sequence[int], mod_seg_stride: int, eps: float = 1e-6):
+    """quant_rows_fp8(ln_modulate_segs(x, ...)) in one pass, bit for bit: out e4m3 [B, R, D] view, out_scale fp32 [B, R]."""
+    x3, q3 = _view3(_dev(x, "ln_segs_fp8.x", BF16), "ln_segs_fp8.x"), _view3(_dev(out, "ln_segs_fp8.out", FP8), "ln_segs_fp8.out")
+    _dev(shift, "ln_segs_fp8.shift", torch.float32), _dev(scale, "ln_segs_fp8.scale", torch.float32)
+    _dev(out_scale, "ln_segs_fp8.out_scale", torch.float32)
+    B, R, D = x3.shape
+    s3 = out_scale if out_scale.dim() == 2 else out_scale.unsqueeze(0)
+    if tuple(q3.shape) != (B, R, D) or tuple(s3.shape) != (B, R) or s3.stride(1) != 1:
+        raise UgError(f"ln_modulate_segs_fp8: out {tuple(out.shape)} / out_scale {tuple(out_scale.shape)} do not match x {tuple(x.shape)}")
+    n = len(seg_bounds) - 1
+    sb = (C.c_int32 * (n + 1))(*[int(v) for v in seg_bounds])
+    check(_lib.load().ug_ln_modulate_segs_fp8(x3.data_ptr(), x3.stride(1), x3.stride(0), q3.data_ptr(), q3.stride(1), q3.stride(0),
+                                              s3.data_ptr(), s3.stride(0), shift.data_ptr(), scale.data_ptr(), shift.stride(0),
+                                              int(mod_seg_stride), n, sb, B, R, D, float(eps), _stream()), "ug_ln_modulate_segs_fp8")
+    return out, out_scale
 
 
 def _slot_mod(t: torch.Tensor, name: str):

@@ -680,6 +680,8 @@ class SequenceParallelUniCombineFlux(UniCombineFlux):
         if not self.sp_enabled:
             return UniCombineFlux.forward(self, hidden_states, condition_latents, condition_ids, condition_types,
                                           encoder_hidden_states, pooled_projections, timestep, img_ids, txt_ids, c_t=c_t, **kwargs)
+        if self.linear_dtype != torch.bfloat16:
+            raise ops.UgError("fp8-quantised block linears (quantize_fp8) are not sharded: run with sp_enabled=False or a bf16 model")
         P, r = self.sp_world, self.sp_rank
         dev = self.device_
         if self._pool is not None:

@@ -23,7 +23,7 @@ import torch
 
 from . import ops
 from .lora_switching_module import LoraLayer
-from .model import BF16, FluxArch, _DoubleBlockW, _SingleBlockW, _TimeTextW, _Weights
+from .model import BF16, FP8, FluxArch, _DoubleBlockW, _SingleBlockW, _TimeTextW, _Weights, quantize_block_linears
 from .ops import UG_ACT_GELU_TANH
 
 DOUBLE_LORA = ("norm1.linear", "attn.to_q", "attn.to_k", "attn.to_v", "attn.to_out.0", "ff.net.2")
@@ -40,6 +40,9 @@ class _LoraPair:
         self.b = torch.zeros(groups, n_sub * n_each, rank, device=device, dtype=BF16)
         self.bw: Optional[torch.Tensor] = None
         self.aw: Optional[torch.Tensor] = None
+        # fp8 operands (UniCombineFlux.quantize_fp8): aw quantised per row (aq, aws) and W2 = bw / w_scale[c] of the linear
+        self.w_scale: Optional[torch.Tensor] = None
+        self.aq = self.aws = self.w2 = None
 
     def build_wide(self):
         """W2 operand of the K-extension form: [n_sub * n_each, groups * 64], block g = B_g with sub-linear j's columns at
@@ -59,6 +62,23 @@ class _LoraPair:
         for g in range(G):
             aw[g * LORA_BLOCK:g * LORA_BLOCK + self.a.shape[1]] = self.a[g]
         self.aw = aw
+        if self.w_scale is not None:
+            self._quantize_operands()
+
+    def quantize_fp8(self, w_scale: torch.Tensor):
+        """Operands of the fp8 form for a linear quantised with per-output-channel scales `w_scale`: the linear's GEMM
+        dequantises its whole accumulator by a_s[r] * w_scale[c], so the K extension carries the update pre-divided —
+        A2 = (x / a_s) A^T (the fp8 masked down-projection of the quantised x with Aq, aws and unit row scales) and
+        W2 = bw / w_scale[c]. Rebuilt in place by build_wide."""
+        self.w_scale = w_scale
+        self.aq = torch.empty(self.aw.shape, device=self.aw.device, dtype=FP8)
+        self.aws = torch.empty(self.aw.shape[0], device=self.aw.device, dtype=torch.float32)
+        self.w2 = torch.empty_like(self.bw)
+        self._quantize_operands()
+
+    def _quantize_operands(self):
+        ops.quant_rows_fp8(self.aw, self.aq, self.aws)
+        self.w2.copy_(self.bw.float() / self.w_scale[:, None])
 
 
 class UniCombineFlux(torch.nn.Module):
@@ -102,6 +122,7 @@ class UniCombineFlux(torch.nn.Module):
         self.overlap_mod_gemv = True  # AdaLN GEMVs (HBM-bound) on a side stream under the tensor-core-bound blocks
         self._side_stream = torch.cuda.Stream(device=self.device_)
         self.add_cond_attn = False  # model_config['add_cond_attn'] (UniCombineTransformerBlock.pyc L201-202)
+        self.linear_dtype = BF16  # float8_e4m3fn after quantize_fp8()
 
     @property
     def dtype(self):
@@ -120,6 +141,9 @@ class UniCombineFlux(torch.nn.Module):
         Every LoRA-wrapped linear gets a `LoraLayer` carrier (`self.lora_layers[name]`: `.active_adapters`, `.scaling`,
         `.set_scale`) for the reference's hooks (unigen_b200.lora_switching_module.enable_lora); `lora_alpha[a]` (default r,
         the UniCombine convention) gives the initial `scaling = lora_alpha / r`, `scaling=` overrides it directly."""
+        if self.linear_dtype != BF16:
+            raise ops.UgError("load_state_dict on an fp8-quantised model: its block linears no longer hold bf16 weights — load the "
+                              "checkpoint into a fresh model, then call quantize_fp8()")
         a, D = self.arch, self.inner_dim
         dev = self.device_
         with torch.no_grad():
@@ -223,6 +247,34 @@ class UniCombineFlux(torch.nn.Module):
                 pair.build_wide()
         self._dirty.clear()
 
+    @torch.no_grad()
+    def quantize_fp8(self):
+        """Opt-in fp8 (e4m3) transformer-block linears, in place; returns self (a second call does nothing). The linears of the
+        double blocks (q|k|v, add_q|k|v, to_out, to_add_out, ff, ff_context) and single blocks (q|k|v, proj_mlp, proj_out) get
+        one fp32 scale per output channel and are stored as e4m3; their bf16 copies are released and leave `state_dict()`. In
+        every forward their operands are quantised per token row on the device (once per operand, shared by the text, image /
+        condition and LoRA GEMMs that read it) and the GEMMs run on the fp8 tensor cores. The switched LoRA update of the
+        quantised linears stays exact in form: its down-projection runs on the quantised operand, and its bf16 K extension is
+        pre-divided by the scales the fp8 GEMM multiplies with (`_LoraPair.quantize_fp8`); the LoRA hooks (`enable_lora`,
+        `set_scale`, `set_adapter`) keep working and rewrite those operands in place. x_embedder and its LoRA, the context /
+        time / text embedders, the AdaLN GEMVs and their LoRA, norm_out / proj_out and attention stay bf16. Call after
+        `load_state_dict`; afterwards `load_state_dict`, `lora_mode="epilogue"` and the sequence-parallel subclass with
+        `sp_enabled=True` raise `UgError`. CUDA graphs captured over
+        this model before the call point at released weights: capture them again."""
+        if self.linear_dtype == FP8:
+            return self
+        if not self.lora:
+            raise ops.UgError("call load_state_dict(..., adapters=..., condition_types=...) before quantize_fp8()")
+        quantize_block_linears(self._ws, self.double + self.single)
+        for i, w in enumerate(self.double):
+            for key, lin in (("qkv", w.qkv), ("to_out", w.to_out), ("ff2", w.ff2)):
+                self.lora[f"transformer_blocks.{i}.{key}"].quantize_fp8(lin[2])
+        for i, w in enumerate(self.single):
+            for key, lin in (("qkv", w.qkv), ("mlp", w.mlp), ("out", w.out)):
+                self.lora[f"single_transformer_blocks.{i}.{key}"].quantize_fp8(lin[2])
+        self.linear_dtype = FP8
+        return self
+
     def lora_modules(self) -> List[LoraLayer]:
         """The LoRA carriers of every switched linear, in registration order — what the reference passes to `enable_lora`."""
         return list(self.lora_layers.values())
@@ -232,6 +284,7 @@ class UniCombineFlux(torch.nn.Module):
         key = (B, S)
         if key in self._bufs:  # one workspace per shape, never freed while the model lives (captured graphs point into them)
             self._buf = self._bufs[key]
+            self._fp8_buffers(self._buf, B, S)
             return self._buf
         D, dev = self.inner_dim, self.device_
         z = lambda *s, dt=BF16: torch.empty(*s, device=dev, dtype=dt)  # noqa: E731
@@ -240,7 +293,17 @@ class UniCombineFlux(torch.nn.Module):
             LT=z(B, S, 3 * self.R, dt=torch.float32), LTW=z(B, S, self.groups * LORA_BLOCK), temb=z(B, D, dt=torch.float32), ctemb=z(B, D, dt=torch.float32),
             tmp=z(B, D, dt=torch.float32), NO=None, mod_plans={},
             rope=z(S, self.arch.attention_head_dim, dt=torch.float32))
+        self._fp8_buffers(self._buf, B, S)
         return self._buf
+
+    def _fp8_buffers(self, buf, B, S):
+        """e4m3 operands (+ one fp32 scale per row) of the quantised block linears: LN output, attention output, FF and CAT.
+        Added to the shape's workspace on its first fp8 forward; the bf16 buffers keep their addresses."""
+        if self.linear_dtype != FP8 or hasattr(buf, "NXQ"):
+            return
+        D, dev = self.inner_dim, self.device_
+        q = lambda w: (torch.empty(B, S, w, device=dev, dtype=FP8), torch.empty(B, S, device=dev, dtype=torch.float32))  # noqa: E731
+        buf.NXQ, buf.AOQ, buf.FFQ, buf.CATQ = q(D), q(D), q(4 * D), q(5 * D)
 
     def _rec(self, name, t):
         if self.trace is not None:
@@ -337,8 +400,27 @@ class UniCombineFlux(torch.nn.Module):
         D = row.shape[-1] // n_chunks
         return [row[:, i * D:(i + 1) * D] for i in range(n_chunks)]
 
-    def _lora_gemm(self, buf, x, w, pair: _LoraPair, seg_bounds, seg_group, out, **kw):
-        """Main GEMM with the switched low-rank update fused into its epilogue."""
+    @staticmethod
+    def _rows(q, lo: int, hi: Optional[int] = None):
+        """Rows [lo, hi) of a quantised operand (e4m3 [B, S, K], scales [B, S]); None stays None (bf16 weight set)."""
+        return None if q is None else (q[0][:, lo:hi], q[1][:, lo:hi])
+
+    def _linear(self, w, x, q, out, **kw):
+        """Plain block linear: the bf16 GEMM of x, or for a quantised (W e4m3, bias, w_scale) the fp8 GEMM of q = (e4m3, scales)."""
+        if len(w) == 3:
+            return ops.gemm_fp8(q[0], q[1], w[0], w[2], out=out, bias=w[1], variant=self.gemm_variant, **kw)
+        return ops.gemm(x, w[0], out=out, bias=w[1], variant=self.gemm_variant, **kw)
+
+    def _lora_gemm(self, buf, x, w, pair: _LoraPair, seg_bounds, seg_group, out, q=None, **kw):
+        """Main GEMM with the switched low-rank update fused into it. A quantised linear (W e4m3, bias, w_scale) takes the
+        quantised operand q = (e4m3 rows, row scales) of x: the masked fp8 down-projection writes (x / a_s) A^T into the K
+        extension, whose W2 is pre-divided by w_scale (see _LoraPair.quantize_fp8)."""
+        if len(w) == 3:
+            tw = buf.LTW[:, :x.shape[1]]
+            ops.gemm_fp8(q[0], None, pair.aq, pair.aws, out=tw, variant=self.gemm_variant,
+                         colmask=dict(block=LORA_BLOCK, seg_bounds=seg_bounds, seg_group=seg_group))
+            return ops.gemm_fp8(q[0], q[1], w[0], w[2], out=out, bias=w[1], variant=self.gemm_variant, a2=tw, w2=pair.w2,
+                                seg_bounds=seg_bounds if kw.get("gate_seg_stride") else None, **kw)
         if self.lora_mode == "mma":
             tw = buf.LTW[:, :x.shape[1]]
             if self.lora_down_mode == "mma" and x.shape[-1] >= 256:
@@ -390,6 +472,9 @@ class UniCombineFlux(torch.nn.Module):
         dev = self.device_
         if list(condition_types) != self.condition_types[:len(condition_types)]:
             raise ops.UgError(f"condition_types {list(condition_types)} do not match the loaded adapters {self.condition_types}")
+        if self.linear_dtype == FP8 and self.lora_mode != "mma":
+            raise ops.UgError(f'lora_mode="{self.lora_mode}" on an fp8-quantised model: its switched update runs as the fp8 GEMM\'s '
+                              'K extension (lora_mode="mma")')
         self._sync_lora()  # scale tables follow the LoRA hooks (lora_switching_module.enable_lora / LoraLayer.set_scale)
         n = len(condition_latents)
         B, N, _ = hidden_states.shape
@@ -431,6 +516,21 @@ class UniCombineFlux(torch.nn.Module):
         L = self.lora
         mp = self._mods(buf, B, n)
         dbl_mods, sgl_mods = mp.dbl, mp.sgl
+        # quantised block linears: one e4m3 operand (+ row scales) per LN output / attention output / FF / CAT, shared by every
+        # GEMM that reads those rows (text, image / condition and LoRA down-projection)
+        fp8 = self.linear_dtype == FP8
+        qn, qa, qf, qc = ((buf.NXQ, buf.AOQ, buf.FFQ, buf.CATQ) if fp8 else (None,) * 4)
+        rows = self._rows
+
+        def ln(shift, scale, seg_bounds, seg_stride):
+            if fp8:
+                ops.ln_modulate_segs_fp8(buf.X, qn[0], qn[1], shift, scale, seg_bounds, seg_stride)
+            else:
+                ops.ln_modulate_segs(buf.X, buf.NX, shift, scale, seg_bounds, seg_stride)
+
+        def quant(x, q):
+            if fp8:
+                ops.quant_rows_fp8(x, q[0], q[1])
 
         for i, w in enumerate(self.double):  # ---- block_forward ----
             p = f"transformer_blocks.{i}"
@@ -440,16 +540,17 @@ class UniCombineFlux(torch.nn.Module):
             m_img = self._chunks(dbl_mods[i][1][0], 6)
             m_c = [self._chunks(dbl_mods[i][1][1 + j], 6) for j in range(n)]
             mods = [m_txt, m_img] + m_c
-            ops.ln_modulate_segs(buf.X, buf.NX, m_txt[0], m_txt[1], bounds, B * 6 * D)
-            ops.gemm(buf.NX[:, :T], w.add_qkv[0], out=buf.QKV[:, :T], bias=w.add_qkv[1], variant=gv, qk_norm=self._qk_norm(buf, w.rms_ctx, 0, T))
+            ln(m_txt[0], m_txt[1], bounds, B * 6 * D)
+            self._linear(w.add_qkv, buf.NX[:, :T], rows(qn, 0, T), buf.QKV[:, :T], qk_norm=self._qk_norm(buf, w.rms_ctx, 0, T))
             self._lora_gemm(buf, buf.NX[:, T:], w.qkv, L[p + ".qkv"], img_cond_bounds, img_cond_groups, buf.QKV[:, T:],
-                            qk_norm=self._qk_norm(buf, w.rms, T, S))
+                            q=rows(qn, T, S), qk_norm=self._qk_norm(buf, w.rms, T, S))
             self._attention(buf, [(0, T, w.rms_ctx), (T, S, w.rms)], "AO", bounds, vis)
-            ops.gemm(buf.AO[:, :T], w.to_add_out[0], out=seg(0), bias=w.to_add_out[1], gate=m_txt[2], residual=seg(0), variant=gv)
+            quant(buf.AO, qa)
+            self._linear(w.to_add_out, buf.AO[:, :T], rows(qa, 0, T), seg(0), gate=m_txt[2], residual=seg(0))
             # to_out[0]: LoRA group AND gate switched per stream inside one launch over [img | c_1 .. c_n]
             if not self.add_cond_attn:
                 self._lora_gemm(buf, buf.AO[:, T:], w.to_out, L[p + ".to_out"], img_cond_bounds, img_cond_groups, buf.X[:, T:],
-                                gate=m_img[2], gate_seg_stride=B * 6 * D, residual=buf.X[:, T:])
+                                q=rows(qa, T, S), gate=m_img[2], gate_seg_stride=B * 6 * D, residual=buf.X[:, T:])
             else:
                 # add_cond_attn (pyc L201-202): the GATED condition attention outputs are also added into the image stream, so
                 # they are materialised once (gated, no residual) and added to both streams
@@ -457,18 +558,20 @@ class UniCombineFlux(torch.nn.Module):
                     raise ops.UgError("add_cond_attn adds condition attention outputs to the image stream: needs Nc == N")
                 g_out = buf.NX[:, T:]  # free until the MLP's LayerNorm pass
                 self._lora_gemm(buf, buf.AO[:, T:], w.to_out, L[p + ".to_out"], img_cond_bounds, img_cond_groups, g_out,
-                                gate=m_img[2], gate_seg_stride=B * 6 * D)
+                                q=rows(qa, T, S), gate=m_img[2], gate_seg_stride=B * 6 * D)
                 ops.add(seg(1), g_out[:, :N], seg(1))
                 for j in range(n):
                     gj = g_out[:, img_cond_bounds[1 + j]:img_cond_bounds[2 + j]]
                     ops.add(seg(2 + j), gj, seg(2 + j))
                     ops.add(seg(1), gj, seg(1))
-            ops.ln_modulate_segs(buf.X, buf.NX, m_txt[3], m_txt[4], bounds, B * 6 * D)
-            ops.gemm(buf.NX[:, :T], w.ffc1[0], out=buf.FF[:, :T], bias=w.ffc1[1], act=UG_ACT_GELU_TANH, variant=gv)
-            ops.gemm(buf.FF[:, :T], w.ffc2[0], out=seg(0), bias=w.ffc2[1], gate=m_txt[5], residual=seg(0), variant=gv)
-            ops.gemm(buf.NX[:, T:], w.ff1[0], out=buf.FF[:, T:], bias=w.ff1[1], act=UG_ACT_GELU_TANH, variant=gv)
+            ln(m_txt[3], m_txt[4], bounds, B * 6 * D)
+            # both up-projections first (disjoint rows of FF), so that one quantisation pass covers FF
+            self._linear(w.ffc1, buf.NX[:, :T], rows(qn, 0, T), buf.FF[:, :T], act=UG_ACT_GELU_TANH)
+            self._linear(w.ff1, buf.NX[:, T:], rows(qn, T, S), buf.FF[:, T:], act=UG_ACT_GELU_TANH)
+            quant(buf.FF, qf)
+            self._linear(w.ffc2, buf.FF[:, :T], rows(qf, 0, T), seg(0), gate=m_txt[5], residual=seg(0))
             self._lora_gemm(buf, buf.FF[:, T:], w.ff2, L[p + ".ff2"], img_cond_bounds, img_cond_groups, buf.X[:, T:],
-                            gate=m_img[5], gate_seg_stride=B * 6 * D, residual=buf.X[:, T:])
+                            q=rows(qf, T, S), gate=m_img[5], gate_seg_stride=B * 6 * D, residual=buf.X[:, T:])
             self._rec(f"double.{i}.hidden", seg(1)); self._rec(f"double.{i}.context", seg(0))
             for j in range(n):
                 self._rec(f"double.{i}.cond{j}", seg(2 + j))
@@ -478,11 +581,13 @@ class UniCombineFlux(torch.nn.Module):
             m_x = self._chunks(sgl_mods[i][0], 3)
             m_c = [self._chunks(sgl_mods[i][1 + j], 3) for j in range(n)]
             mods = [m_x] + m_c
-            ops.ln_modulate_segs(buf.X, buf.NX, m_x[0], m_x[1], all_bounds, B * 3 * D)
-            self._lora_gemm(buf, buf.NX, w.qkv, L[p + ".qkv"], all_bounds, all_groups, buf.QKV, qk_norm=self._qk_norm(buf, w.rms, 0, S))
-            self._lora_gemm(buf, buf.NX, w.mlp, L[p + ".mlp"], all_bounds, all_groups, buf.CAT[:, :, D:], act=UG_ACT_GELU_TANH)
+            ln(m_x[0], m_x[1], all_bounds, B * 3 * D)
+            self._lora_gemm(buf, buf.NX, w.qkv, L[p + ".qkv"], all_bounds, all_groups, buf.QKV, q=qn,
+                            qk_norm=self._qk_norm(buf, w.rms, 0, S))
+            self._lora_gemm(buf, buf.NX, w.mlp, L[p + ".mlp"], all_bounds, all_groups, buf.CAT[:, :, D:], q=qn, act=UG_ACT_GELU_TANH)
             self._attention(buf, [(0, S, w.rms)], "CAT", bounds, vis)
-            self._lora_gemm(buf, buf.CAT, w.out, L[p + ".out"], all_bounds, all_groups, buf.X, gate=m_x[2],
+            quant(buf.CAT, qc)
+            self._lora_gemm(buf, buf.CAT, w.out, L[p + ".out"], all_bounds, all_groups, buf.X, q=qc, gate=m_x[2],
                             gate_seg_stride=B * 3 * D, residual=buf.X)
             self._rec(f"single.{i}.hidden", buf.X[:, :T + N])
             for j in range(n):
