@@ -113,16 +113,25 @@ class _SingleBlockW:
 
 def quantize_block_linears(ws: _Weights, blocks) -> None:
     """Every linear named in a block's FP8_LINEARS becomes (W e4m3 [N, K], bias bf16 [N], w_scale fp32 [N]), one scale per output
-    channel; the bf16 weight is released and its state-dict views are dropped (the bias stays). Marks the blocks `fp8`."""
+    channel; the bf16 weight is released and its state-dict views are dropped (the bias stays). Marks the blocks `fp8`.
+    A dotted name reaches a linear of a sub-object (`attn.qkv`); a linear or sub-object that is None (absent in this block
+    layout, e.g. `to_add_out` of a context_pre_only block) is skipped."""
     views = ws.views
     for w in blocks:
         for name in w.FP8_LINEARS:
-            W, bias = getattr(w, name)
+            *path, attr = name.split(".")
+            owner = w
+            for p in path:
+                owner = getattr(owner, p) if owner is not None else None
+            lin = getattr(owner, attr) if owner is not None else None
+            if lin is None:
+                continue
+            W, bias = lin
             q, w_scale = ops.quant_rows_fp8(W)  # a row of W is an output channel
             ptr = W.untyped_storage().data_ptr()
             for k in [k for k, v in views.items() if k.endswith(".weight") and v.untyped_storage().data_ptr() == ptr]:
                 del views[k]
-            setattr(w, name, (q, bias, w_scale))
+            setattr(owner, attr, (q, bias, w_scale))
         w.fp8 = True
 
 
@@ -164,6 +173,7 @@ class _DenoiserBase(torch.nn.Module):
         self.fuse_qk_norm = True
         self.trace: Optional[Dict[str, torch.Tensor]] = None  # set to {} to record per-block intermediates
         self.clone_outputs = True  # forward returns copies, not views of the workspace / graph-static buffers
+        self.linear_dtype = BF16  # float8_e4m3fn after quantize_fp8()
 
     @property
     def dtype(self):
@@ -180,6 +190,9 @@ class _DenoiserBase(torch.nn.Module):
         return iter(self._ws.views.values())
 
     def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):
+        if self.linear_dtype != BF16:
+            raise ops.UgError("load_state_dict on an fp8-quantised model: its block linears no longer hold bf16 weights — load the "
+                              "checkpoint into a fresh model, then call quantize_fp8()")
         missing = [k for k in self._ws.views if k not in state_dict]
         unexpected = [k for k in state_dict if k not in self._ws.views]
         if strict and (missing or unexpected):
@@ -201,6 +214,9 @@ class _DenoiserBase(torch.nn.Module):
     def init_random_(self, seed: int = 0, zero_linear_std: Optional[float] = 0.02):
         """nn.Linear / nn.Conv2d default init directly on the device (bench: the 18.7 B Flux parameters never exist on
         the host). Zero-linears (`controlnet_add_*`) get N(0, zero_linear_std), or true zeros for None."""
+        if self.linear_dtype != BF16:
+            raise ops.UgError("init_random_ on an fp8-quantised model: its quantised block weights are not in state_dict() any more "
+                              "and would keep their values — initialise a fresh model, then call quantize_fp8()")
         gen = torch.Generator(device=self.device_).manual_seed(seed)
         for k, v in self._ws.views.items():
             if k.endswith(".pos_embed"):
@@ -242,6 +258,44 @@ class _DenoiserBase(torch.nn.Module):
     def _rec(self, name: str, t: torch.Tensor):
         if self.trace is not None:
             self.trace[name] = t.detach().float().clone()
+
+    def _fp8_blocks(self) -> list:
+        """The blocks whose FP8_LINEARS `quantize_fp8()` converts (the model's base and control transformer blocks)."""
+        raise NotImplementedError
+
+    @torch.no_grad()
+    def _quantize_fp8(self):
+        """What every model's `quantize_fp8()` does: quantise the linears of `_fp8_blocks()` in place (once), then drop the
+        workspaces and every CUDA graph captured over them — the pipeline's whole-loop graphs included — since they hold bf16
+        operands only and point at the released weights."""
+        if not self._control_ready:
+            raise ops.UgError("call init_condition_block(condition_nums=..., control_params=...) before quantize_fp8()")
+        if self.linear_dtype == FP8:
+            return self
+        quantize_block_linears(self._ws, self._fp8_blocks())
+        self.linear_dtype = FP8
+        from .pipeline import _GRAPHS_ATTR
+        self.__dict__.pop(_GRAPHS_ATTR, None)
+        self._workspaces.clear()
+        self._graphs.clear()
+        self._buf = None
+        return self
+
+    def _ln(self, w, x, nx, q, shift, scale):
+        """LN + modulate of a block input into the bf16 operand `nx`, or (fp8 weight set) straight into q = (e4m3, row scales)."""
+        if w.fp8:
+            ops.ln_modulate_fp8(x, q[0], q[1], shift, scale)
+        else:
+            ops.ln_modulate(x, nx, shift, scale)
+
+    def _linear(self, wl, x, q, out, quantize: bool = False, **epi):
+        """One block linear: the bf16 GEMM of x with (W, bias), or for an fp8 (W e4m3, bias, w_scale) the fp8 GEMM of
+        q = (e4m3 rows, row scales) — quantised from x first when `quantize` (operands no LN kernel produced)."""
+        if len(wl) == 3:
+            if quantize:
+                ops.quant_rows_fp8(x, q[0], q[1])
+            return ops.gemm_fp8(q[0], q[1], wl[0], wl[2], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
+        return ops.gemm(x, wl[0], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
 
     def _cached_workspace(self, key, make):
         """Workspace for input shape `key` (built by `make()` on first use). Buffers of a shape stay where they are for as
@@ -329,7 +383,6 @@ class UniGenFlux(_DenoiserBase):
         self.norm_out_w = ws.linear("norm_out.linear", 2 * D, D)
         # proj_out has only in_channels (64) output features: keep it as is, the GEMM masks the partial N tile
         self.proj_out_w = ws.linear("proj_out", a.in_channels, D)
-        self.linear_dtype = BF16  # float8_e4m3fn after quantize_fp8()
 
     # ---------------------------------------------------------------------------------------------------------
     # reference API: construction
@@ -386,19 +439,6 @@ class UniGenFlux(_DenoiserBase):
             raise ops.UgError("the B200-native path is forward-only (SURVEY.md §3.2: training is out of scope)")
         return self
 
-    def load_state_dict(self, state_dict, strict: bool = True, assign: bool = False):
-        if self.linear_dtype != BF16:
-            raise ops.UgError("load_state_dict on an fp8-quantised model: its block linears no longer hold bf16 weights — load the "
-                              "checkpoint into a fresh model, then call quantize_fp8()")
-        return super().load_state_dict(state_dict, strict=strict, assign=assign)
-
-    def init_random_(self, seed: int = 0, zero_linear_std: Optional[float] = 0.02):
-        if self.linear_dtype != BF16:
-            raise ops.UgError("init_random_ on an fp8-quantised model: its quantised block weights are not in state_dict() any more "
-                              "and would keep their values — initialise a fresh model, then call quantize_fp8()")
-        return super().init_random_(seed=seed, zero_linear_std=zero_linear_std)
-
-    @torch.no_grad()
     def quantize_fp8(self):
         """Opt-in fp8 (e4m3) transformer-block linears, in place; returns self. Every linear of the base and control double
         blocks (q|k|v, add_q|k|v, to_out, to_add_out, ff, ff_context) and single blocks (q|k|v, proj_mlp, proj_out) gets one fp32
@@ -408,19 +448,10 @@ class UniGenFlux(_DenoiserBase):
         add-linears, proj_out and attention stay bf16. Call after `from_pretrained` / `init_condition_block` and any
         `load_state_dict`. Afterwards `state_dict()` / `parameters()` no longer list the quantised weights (their biases and every
         bf16 tensor stay), and `load_state_dict` / `init_random_` raise `UgError`."""
-        if not self._control_ready:
-            raise ops.UgError("call init_condition_block(condition_nums=..., control_params=...) before quantize_fp8()")
-        if self.linear_dtype == FP8:
-            return self
-        quantize_block_linears(self._ws, self.double + self.ctrl_double + self.single + self.ctrl_single)
-        self.linear_dtype = FP8
-        # workspaces (and the graphs captured over them, the pipeline's whole-loop graphs included) hold bf16 operands only
-        from .pipeline import _GRAPHS_ATTR
-        self.__dict__.pop(_GRAPHS_ATTR, None)
-        self._workspaces.clear()
-        self._graphs.clear()
-        self._buf = None
-        return self
+        return self._quantize_fp8()
+
+    def _fp8_blocks(self):
+        return self.double + self.ctrl_double + self.single + self.ctrl_single
 
     def init_condition_block(self, condition_nums: int = 1, **kwargs):
         """reference src/UniGenTransformer.py:713-715 -> init_control_block(kwargs['control_params'])."""
@@ -658,22 +689,6 @@ class UniGenFlux(_DenoiserBase):
             if n_smp:
                 ops.qk_rmsnorm_rope(qk[:, n_ctx:], 2 * H, dh, rms_smp, rope[n_ctx:S] if rope is not None else None, heads_per_weight=H)
         return self._attend(buf, S, buf.AO[:, :S])
-
-    def _ln(self, w, x, nx, q, shift, scale):
-        """LN + modulate of a block input into the bf16 operand `nx`, or (fp8 weight set) straight into q = (e4m3, row scales)."""
-        if w.fp8:
-            ops.ln_modulate_fp8(x, q[0], q[1], shift, scale)
-        else:
-            ops.ln_modulate(x, nx, shift, scale)
-
-    def _linear(self, wl, x, q, out, quantize: bool = False, **epi):
-        """One block linear: the bf16 GEMM of x with (W, bias), or for an fp8 (W e4m3, bias, w_scale) the fp8 GEMM of
-        q = (e4m3 rows, row scales) — quantised from x first when `quantize` (operands no LN kernel produced)."""
-        if len(wl) == 3:
-            if quantize:
-                ops.quant_rows_fp8(x, q[0], q[1])
-            return ops.gemm_fp8(q[0], q[1], wl[0], wl[2], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
-        return ops.gemm(x, wl[0], out=out, bias=wl[1], variant=self.gemm_variant, **epi)
 
     def _double_block(self, buf, w: _DoubleBlockW, mod_smp, mod_ctx, smp_in, ctx_in, smp_out, ctx_out, rope):
         """diffusers FluxTransformerBlock (SURVEY.md §A.2). smp/ctx = image-role / text-role streams ([B, n, D] views);

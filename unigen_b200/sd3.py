@@ -35,7 +35,7 @@ from typing import Any, Dict, Optional
 import torch
 
 from . import ops
-from .model import BF16, _DenoiserBase, _TimeTextW, _Weights
+from .model import BF16, FP8, _DenoiserBase, _TimeTextW, _Weights
 from .ops import UG_ACT_GELU_TANH
 
 
@@ -118,6 +118,11 @@ class _AttnW:
 
 class _JointBlockW:
     """JointTransformerBlock(dim, heads, head_dim, context_pre_only, qk_norm, use_dual_attention) parameters."""
+    # linears `UniGenSD3.quantize_fp8()` converts (model.quantize_block_linears); the ones a block layout lacks (attn2 without
+    # dual attention, to_add_out / ff_context in a context_pre_only block) are None and skipped
+    FP8_LINEARS = ("attn.qkv", "attn.add_qkv", "attn.to_out", "attn.to_add_out", "attn2.qkv", "attn2.to_out",
+                   "ff1", "ff2", "ffc1", "ffc2")
+    fp8 = False
 
     def __init__(self, ws: _Weights, p: str, D: int, dh: int, dual: bool, context_pre_only: bool, qk_norm: bool):
         self.dual, self.context_pre_only = dual, context_pre_only
@@ -259,6 +264,9 @@ class UniGenSD3(_DenoiserBase):
         context_pre_only (`norm1_context.linear` [2D, D], no `to_add_out` / `ff_context`) while its control twin is not
         ([6D, D]) — `strict=False` does not forgive a size mismatch, so the reference call raises RuntimeError with the
         shipped 24 + 24 layout; here keys whose shapes differ are skipped and the call succeeds."""
+        if self.linear_dtype != BF16:
+            raise ops.UgError("init_control_param on an fp8-quantised model: it copies through the state-dict views, which no longer "
+                              "list the quantised block weights — call it (or use_transformer_params) before quantize_fp8()")
         v = self._ws.views
 
         def copy_prefix(dst: str, src: str):
@@ -273,6 +281,22 @@ class UniGenSD3(_DenoiserBase):
         for j in range(min(self.control_blocks_num, self.arch.num_layers)):
             copy_prefix(f"control_transformer_blocks.{j}", f"transformer_blocks.{j}")
         self._weights_loaded()
+
+    def quantize_fp8(self):
+        """Opt-in fp8 (e4m3) transformer-block linears, in place; returns self (a second call does nothing). Every linear of the
+        base and control joint blocks — q|k|v, add_q|k|v, to_out, to_add_out, attn2 q|k|v and attn2.to_out (dual-attention
+        layers), ff and ff_context (the context_pre_only last block has neither to_add_out nor ff_context) — gets one fp32 scale
+        per output channel and is stored as e4m3; its bf16 copy is released (and leaves `state_dict()`). In every forward their
+        operands are quantised per token row on the device and the GEMMs run on the fp8 tensor cores. The patch / context /
+        time / text embedders, the AdaLN GEMVs, the control add-linears, norm_out / proj_out, attention and the whole CoMoE
+        pre-stage (routed experts, shared experts, gate: routing stays bit-exact) stay bf16. Call after `init_condition_block`
+        and any `load_state_dict` / `init_control_param`. Afterwards `state_dict()` / `parameters()` no longer list the quantised
+        weights (their biases and every bf16 tensor stay), and `load_state_dict`, `init_random_` and `init_control_param`
+        raise `UgError`."""
+        return self._quantize_fp8()
+
+    def _fp8_blocks(self):
+        return self.blocks + self.ctrl_blocks
 
     def _weights_loaded(self):
         self.pos_embed_w._crop.clear()
@@ -302,6 +326,15 @@ class UniGenSD3(_DenoiserBase):
             PAT=z(B, N, kpe), NO=z(B, N, D), OUT=z(B, N, a.patch_size ** 2 * a.out_channels), capacity=C)
         if self.use_modulate:  # per-sample, per-expert modulation vectors of the two linear experts
             b.MODC, b.MODH = z(B, E, D, dt=torch.float32), z(B, E, D, dt=torch.float32)
+        if self.linear_dtype == FP8:
+            # e4m3 operands (+ one fp32 scale per row) of the quantised block linears. Only base and control blocks are
+            # quantised, and they run over N + T rows (the 2N + T rows of shared_expert[1] stay bf16). Row layout as in
+            # NX / NX2 / AO / FF: sample rows [0, n), context rows [n, n + T).
+            f8 = lambda *sh: z(*sh, dt=FP8)  # noqa: E731
+            b.NXQ, b.NXS = f8(B, S, D), z(B, S, dt=torch.float32)
+            b.NX2Q, b.NX2S = f8(B, N, D), z(B, N, dt=torch.float32)
+            b.AOQ, b.AOS = f8(B, S, D), z(B, S, dt=torch.float32)
+            b.FFQ, b.FFS = f8(B, S, 4 * D), z(B, S, dt=torch.float32)
         return b
 
     def _sd3_mod_plans(self, buf, B: int):
@@ -342,15 +375,16 @@ class UniGenSD3(_DenoiserBase):
         ops.gemm(pat, w.w, out=out, bias=w.b, residual=table.unsqueeze(0).expand(B, -1, -1), variant=self.gemm_variant)
         return out
 
-    def _attn_qkv(self, x, aw_qkv, rms, qkv_rows):
-        """q|k|v projection of one stream into its rows of a fused QKV buffer + in-place per-head RMSNorm (no RoPE)."""
+    def _attn_qkv(self, x, q, aw_qkv, rms, qkv_rows):
+        """q|k|v projection of one stream into its rows of a fused QKV buffer + in-place per-head RMSNorm (no RoPE). For an
+        fp8 linear, q = (e4m3 rows, row scales) of x is the GEMM operand."""
         a = self.arch
         if rms is not None and self.fuse_qk_norm and x.dim() == 3 and aw_qkv[0].dim() == 2:
             # per-head RMSNorm of q / k inside the projection GEMM's epilogue (fp32 accumulator, no second pass over the buffer)
-            ops.gemm(x, aw_qkv[0], out=qkv_rows, bias=aw_qkv[1], variant=self.gemm_variant,
-                     qk_norm=dict(weight=rms, head_dim=a.attention_head_dim, d=self.inner_dim, cos_sin=None, eps=1e-6))
+            self._linear(aw_qkv, x, q, out=qkv_rows,
+                         qk_norm=dict(weight=rms, head_dim=a.attention_head_dim, d=self.inner_dim, cos_sin=None, eps=1e-6))
             return
-        ops.gemm(x, aw_qkv[0], out=qkv_rows, bias=aw_qkv[1], variant=self.gemm_variant)
+        self._linear(aw_qkv, x, q, out=qkv_rows)
         if rms is not None:
             ops.qk_rmsnorm_rope(qkv_rows[:, :, :2 * self.inner_dim], 2 * a.num_attention_heads, a.attention_head_dim, rms, None,
                                 heads_per_weight=a.num_attention_heads)
@@ -359,12 +393,23 @@ class UniGenSD3(_DenoiserBase):
         """JointTransformerBlock.forward (src/UniGenUtils.py:440-522) + JointAttnProcessor2_0 (sample-first joint attention).
         smp/ctx = sample / context streams ([B, n, D] views); outputs may alias inputs. ctx_out=None skips the context
         stream's post-attention half: exact for context_pre_only blocks and whenever the caller discards the context output
-        (control blocks: `encoder_hidden_states` is re-read from moe_output every call, src/UniGenTransformer.py:566)."""
+        (control blocks: `encoder_hidden_states` is re-read from moe_output every call, src/UniGenTransformer.py:566).
+        An fp8 weight set (`w.fp8`, after quantize_fp8) runs its linears on e4m3 operands: every LayerNorm-modulate writes
+        e4m3 rows + row scales directly, AO / AO2 / FF are quantised once per stream before their down-projection. The
+        weight set decides, not a model flag: the bf16 shared experts of the pre-stage run through here unchanged."""
         a, D = self.arch, self.inner_dim
         H, dh = a.num_attention_heads, a.attention_head_dim
         B, n_smp, n_ctx = smp_in.shape[0], smp_in.shape[1], ctx_in.shape[1]
         S = n_smp + n_ctx
-        gv = self.gemm_variant
+        qn_s = qn_c = qn2 = qa_s = qa_c = qf_s = qf_c = None
+        if w.fp8:
+            # Everything below runs on one stream, in program order, and the two streams own disjoint rows of every buffer.
+            # Reuses: NXQ's sample / context rows take the second LN of their stream once q|k|v (their first consumer) has
+            # run; AOQ's sample rows take AO2 once to_out has read AO; FFQ is written by the GEMM right before its only reader.
+            qn_s, qn_c = (buf.NXQ[:, :n_smp], buf.NXS[:, :n_smp]), (buf.NXQ[:, n_smp:S], buf.NXS[:, n_smp:S])
+            qn2 = (buf.NX2Q[:, :n_smp], buf.NX2S[:, :n_smp])
+            qa_s, qa_c = (buf.AOQ[:, :n_smp], buf.AOS[:, :n_smp]), (buf.AOQ[:, n_smp:S], buf.AOS[:, n_smp:S])
+            qf_s, qf_c = (buf.FFQ[:, :n_smp], buf.FFS[:, :n_smp]), (buf.FFQ[:, n_smp:S], buf.FFS[:, n_smp:S])
         if w.dual:
             sh_a, sc_a, g_a, sh_m, sc_m, g_m, sh_a2, sc_a2, g_a2 = mod_smp
         else:
@@ -374,28 +419,28 @@ class UniGenSD3(_DenoiserBase):
         else:
             csh_a, csc_a, cg_a, csh_m, csc_m, cg_m = mod_ctx
         nx_s, nx_c = buf.NX[:, :n_smp], buf.NX[:, n_smp:S]
-        ops.ln_modulate(smp_in, nx_s, sh_a, sc_a)
+        self._ln(w, smp_in, nx_s, qn_s, sh_a, sc_a)
         if w.dual:  # norm_hidden_states2 of the block INPUT (before any residual update, which may be in place)
-            ops.ln_modulate(smp_in, buf.NX2[:, :n_smp], sh_a2, sc_a2)
-        ops.ln_modulate(ctx_in, nx_c, csh_a, csc_a)
-        self._attn_qkv(nx_s, w.attn.qkv, w.attn.rms, buf.QKV[:, :n_smp])
-        self._attn_qkv(nx_c, w.attn.add_qkv, w.attn.rms_ctx, buf.QKV[:, n_smp:S])
+            self._ln(w, smp_in, buf.NX2[:, :n_smp], qn2, sh_a2, sc_a2)
+        self._ln(w, ctx_in, nx_c, qn_c, csh_a, csc_a)
+        self._attn_qkv(nx_s, qn_s, w.attn.qkv, w.attn.rms, buf.QKV[:, :n_smp])
+        self._attn_qkv(nx_c, qn_c, w.attn.add_qkv, w.attn.rms_ctx, buf.QKV[:, n_smp:S])
         ao = buf.AO[:, :S]
         ops.attention(buf.QKV[:, :S, 0:D], buf.QKV[:, :S, D:2 * D], buf.QKV[:, :S, 2 * D:3 * D], ao, H, dh, variant=self.attn_variant)
-        ops.gemm(ao[:, :n_smp], w.attn.to_out[0], out=smp_out, bias=w.attn.to_out[1], gate=g_a, residual=smp_in, variant=gv)
+        self._linear(w.attn.to_out, ao[:, :n_smp], qa_s, out=smp_out, quantize=True, gate=g_a, residual=smp_in)
         if w.dual:
-            self._attn_qkv(buf.NX2[:, :n_smp], w.attn2.qkv, w.attn2.rms, buf.QKV2[:, :n_smp])
+            self._attn_qkv(buf.NX2[:, :n_smp], qn2, w.attn2.qkv, w.attn2.rms, buf.QKV2[:, :n_smp])
             q2 = buf.QKV2[:, :n_smp]
             ops.attention(q2[:, :, 0:D], q2[:, :, D:2 * D], q2[:, :, 2 * D:3 * D], buf.AO2[:, :n_smp], H, dh, variant=self.attn_variant)
-            ops.gemm(buf.AO2[:, :n_smp], w.attn2.to_out[0], out=smp_out, bias=w.attn2.to_out[1], gate=g_a2, residual=smp_out, variant=gv)
-        ops.ln_modulate(smp_out, nx_s, sh_m, sc_m)
-        ops.gemm(nx_s, w.ff1[0], out=buf.FF[:, :n_smp], bias=w.ff1[1], act=UG_ACT_GELU_TANH, variant=gv)
-        ops.gemm(buf.FF[:, :n_smp], w.ff2[0], out=smp_out, bias=w.ff2[1], gate=g_m, residual=smp_out, variant=gv)
+            self._linear(w.attn2.to_out, buf.AO2[:, :n_smp], qa_s, out=smp_out, quantize=True, gate=g_a2, residual=smp_out)
+        self._ln(w, smp_out, nx_s, qn_s, sh_m, sc_m)
+        self._linear(w.ff1, nx_s, qn_s, out=buf.FF[:, :n_smp], act=UG_ACT_GELU_TANH)
+        self._linear(w.ff2, buf.FF[:, :n_smp], qf_s, out=smp_out, quantize=True, gate=g_m, residual=smp_out)
         if ctx_out is not None and not w.context_pre_only:
-            ops.gemm(ao[:, n_smp:S], w.attn.to_add_out[0], out=ctx_out, bias=w.attn.to_add_out[1], gate=cg_a, residual=ctx_in, variant=gv)
-            ops.ln_modulate(ctx_out, nx_c, csh_m, csc_m)
-            ops.gemm(nx_c, w.ffc1[0], out=buf.FF[:, n_smp:S], bias=w.ffc1[1], act=UG_ACT_GELU_TANH, variant=gv)
-            ops.gemm(buf.FF[:, n_smp:S], w.ffc2[0], out=ctx_out, bias=w.ffc2[1], gate=cg_m, residual=ctx_out, variant=gv)
+            self._linear(w.attn.to_add_out, ao[:, n_smp:S], qa_c, out=ctx_out, quantize=True, gate=cg_a, residual=ctx_in)
+            self._ln(w, ctx_out, nx_c, qn_c, csh_m, csc_m)
+            self._linear(w.ffc1, nx_c, qn_c, out=buf.FF[:, n_smp:S], act=UG_ACT_GELU_TANH)
+            self._linear(w.ffc2, buf.FF[:, n_smp:S], qf_c, out=ctx_out, quantize=True, gate=cg_m, residual=ctx_out)
 
     def _expert_branch(self, buf, br: int, route, B: int, N: int):
         """All E experts of one branch: SD3SingleTransformerBlock (src/UniGenUtils.py:386-414) on the [E*C, D] slot buffer
