@@ -549,7 +549,8 @@ int ug_im2col_bf16(const void* x, int32_t x_is_f32, int64_t sb, int64_t sy, int6
                    int32_t h_out, int32_t w_out, int32_t k_pad, float alpha, float beta, void* stream);
 
 /* GroupNorm(groups, c, eps, affine) [+ SiLU] over NHWC bf16 [batch, pixels, c]: statistics in fp32, deterministic (no atomics):
- * per-block partial sums -> fixed-order fold -> normalise / scale / shift / activate (three launches). `stats`: fp32 scratch of
+ * per-block sums shifted by a pivot from the image (no cancellation when the mean is large against the spread) -> fixed-order
+ * merge of the blocks' (mean, M2) pairs -> normalise / scale / shift / activate (three launches). `stats`: fp32 scratch of
  * batch * groups * 2 * (1 + UG_GROUPNORM_MAX_CHUNKS) elements. y may alias x. */
 #define UG_GROUPNORM_MAX_CHUNKS 1024
 int ug_groupnorm_bf16(const void* x, void* y, const void* gamma, const void* beta, float* stats, int32_t batch, int32_t pixels,

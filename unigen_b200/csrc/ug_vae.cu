@@ -25,11 +25,18 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
 
 // ---------------------------------------------------------------------------------------------------------------------
 // GroupNorm statistics, deterministic (no floating-point atomics: the same input gives the same bits on every run, eager or graph
-// replay). Pass 1: grid (chunks, batch); a block walks its share of the pixels, thread t owns the channel octet t % (c / 8) of
-// every (t / (c / 8))-th pixel; the per-thread sums are folded over the pixel lanes, then over each group's channels, in a fixed
-// order, and the block writes one (sum, sum of squares) pair per group. Pass 2: one warp per (image, group) folds the blocks'
-// pairs in a fixed order.
+// replay). Every sum is taken of x - P, P = the group's first channel at the image's first pixel (a bf16 value, so x - P is exact
+// in fp32): a one-pass E[x^2] - mean^2 cancels all its digits once the group's mean is ~1e3 x its spread, the shifted sums only
+// lose the digits of (mean - P)^2 / var, which is O(1) for a pivot drawn from the data.
+// Pass 1: grid (chunks, batch); a block walks its share of the pixels, thread t owns the channel octet t % (c / 8) of every
+// (t / (c / 8))-th pixel; the per-thread shifted sums are folded over the pixel lanes, then over each group's channels, in a fixed
+// order, and the block writes one (mean - P, M2) pair per group (its element count follows from the block index).
+// Pass 2: one warp per (image, group) merges the blocks' pairs with Chan's formula in a fixed order and stores (mean, var).
 // ---------------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float groupnorm_pivot(const __nv_bfloat16* x, long long b, int pixels, int c, int cpg, int ch) {
+  return __bfloat162float(x[b * pixels * c + (ch / cpg) * cpg]);
+}
+
 __global__ void __launch_bounds__(256) groupnorm_partial_kernel(const __nv_bfloat16* __restrict__ x, float* __restrict__ partial,
                                                                 int pixels, int c, int groups) {
   __shared__ float part[256][17];  // [thread][8 sums | 8 sums of squares] (+1: no bank conflicts on the column walk)
@@ -40,9 +47,12 @@ __global__ void __launch_bounds__(256) groupnorm_partial_kernel(const __nv_bfloa
   const int lanes_px = blockDim.x / octets;  // pixels a block covers per sweep (host guarantees octets <= blockDim.x)
   const int o = threadIdx.x % octets, sub = threadIdx.x / octets;
   const int per_block = (pixels + gridDim.x - 1) / gridDim.x;
-  const int p0 = blockIdx.x * per_block, p1 = min(pixels, p0 + per_block);
+  const int p0 = min(pixels, blockIdx.x * per_block), p1 = min(pixels, p0 + per_block);
   float s[8] = {0, 0, 0, 0, 0, 0, 0, 0}, q[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   if (sub < lanes_px) {
+    float pv[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) pv[i] = groupnorm_pivot(x, b, pixels, c, cpg, o * 8 + i);
     const __nv_bfloat16* base = x + ((long long)b * pixels) * c + o * 8;
     int p = p0 + sub;
     // four pixels per trip: four independent 16-byte loads in flight per thread (the pass is a pure HBM stream)
@@ -56,8 +66,9 @@ __global__ void __launch_bounds__(256) groupnorm_partial_kernel(const __nv_bfloa
         unpack8(v[u], f);
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          s[i] += f[i];
-          q[i] = fmaf(f[i], f[i], q[i]);
+          const float t = f[i] - pv[i];
+          s[i] += t;
+          q[i] = fmaf(t, t, q[i]);
         }
       }
     }
@@ -67,8 +78,9 @@ __global__ void __launch_bounds__(256) groupnorm_partial_kernel(const __nv_bfloa
       unpack8(v, f);
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
-        s[i] += f[i];
-        q[i] = fmaf(f[i], f[i], q[i]);
+        const float t = f[i] - pv[i];
+        s[i] += t;
+        q[i] = fmaf(t, t, q[i]);
       }
     }
   }
@@ -89,39 +101,56 @@ __global__ void __launch_bounds__(256) groupnorm_partial_kernel(const __nv_bfloa
     chq[ch] = qq;
   }
   __syncthreads();
+  const float n = (float)(p1 - p0) * (float)cpg;
   for (int g = threadIdx.x; g < groups; g += blockDim.x) {
     float ss = 0.0f, qq = 0.0f;
     for (int j = 0; j < cpg; ++j) {
       ss += chs[g * cpg + j];
       qq += chq[g * cpg + j];
     }
+    const float m = n > 0.0f ? ss / n : 0.0f;
     float* dst = partial + (((long long)b * gridDim.x + blockIdx.x) * groups + g) * 2;
-    dst[0] = ss;
-    dst[1] = qq;
+    dst[0] = m;
+    dst[1] = fmaxf(fmaf(-ss, m, qq), 0.0f);
   }
 }
 
-__global__ void __launch_bounds__(32) groupnorm_finalize_kernel(const float* __restrict__ partial, float* __restrict__ stats, int chunks,
-                                                                int groups) {
+// Chan et al.: (n_a, m_a, M2_a) += (n_b, m_b, M2_b); an empty side leaves the other unchanged
+__device__ __forceinline__ void chan_merge(float& n, float& m, float& m2, float nb, float mb, float m2b) {
+  const float nt = n + nb;
+  if (nb == 0.0f || nt == 0.0f) return;
+  const float d = mb - m, f = nb / nt;
+  m = fmaf(d, f, m);
+  m2 = m2 + m2b + d * d * n * f;
+  n = nt;
+}
+
+__global__ void __launch_bounds__(32) groupnorm_finalize_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ partial,
+                                                                float* __restrict__ stats, int chunks, int pixels, int c, int groups) {
   const int b = blockIdx.x / groups, g = blockIdx.x % groups;
-  float ss = 0.0f, qq = 0.0f;
+  const int cpg = c / groups;
+  const int per_block = (pixels + chunks - 1) / chunks;
+  float n = 0.0f, m = 0.0f, m2 = 0.0f;
   for (int k = threadIdx.x; k < chunks; k += 32) {
     const float* src = partial + (((long long)b * chunks + k) * groups + g) * 2;
-    ss += src[0];
-    qq += src[1];
+    const int p0 = min(pixels, k * per_block), p1 = min(pixels, p0 + per_block);
+    chan_merge(n, m, m2, (float)(p1 - p0) * (float)cpg, src[0], src[1]);
   }
-  for (int off = 16; off > 0; off >>= 1) {
-    ss += __shfl_xor_sync(0xffffffffu, ss, off);
-    qq += __shfl_xor_sync(0xffffffffu, qq, off);
+  for (int off = 1; off < 32; off <<= 1) {
+    const float nb = __shfl_xor_sync(0xffffffffu, n, off), mb = __shfl_xor_sync(0xffffffffu, m, off),
+                m2b = __shfl_xor_sync(0xffffffffu, m2, off);
+    chan_merge(n, m, m2, nb, mb, m2b);
   }
   if (threadIdx.x == 0) {
-    stats[((long long)b * groups + g) * 2] = ss;
-    stats[((long long)b * groups + g) * 2 + 1] = qq;
+    stats[((long long)b * groups + g) * 2] = groupnorm_pivot(x, b, pixels, c, cpg, g * cpg) + m;
+    stats[((long long)b * groups + g) * 2 + 1] = m2 / n;
   }
 }
 
 // Normalise + affine (+ SiLU). The grid stride is a multiple of c / 8, so a thread keeps ONE channel octet for its whole walk:
-// its eight (scale, shift) pairs  a = rstd * gamma, d = beta - mean * a  are rebuilt only when the walk crosses into the next image.
+// its eight (mean, a = rstd * gamma) pairs are rebuilt only when the walk crosses into the next image. y = (x - mean) * a + beta:
+// x - mean is exact when x is near the mean, where the folded form x * a + (beta - mean * a) would round beta - mean * a at the
+// scale of mean * a.
 template <bool kSilu>
 __global__ void __launch_bounds__(256, 3) groupnorm_apply_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y,
                                                               const __nv_bfloat16* __restrict__ gamma,
@@ -129,33 +158,33 @@ __global__ void __launch_bounds__(256, 3) groupnorm_apply_kernel(const __nv_bflo
                                                               int pixels, int c, int groups, float eps, long long total_octets) {
   const int octets = c >> 3;
   const int cpg = c / groups;
-  const float inv_n = 1.0f / ((float)pixels * (float)cpg);
   const long long stride = (long long)gridDim.x * blockDim.x;
   const long long per_image = (long long)pixels * octets;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int o = (int)(i % octets);
-  float gm[8], bt[8], a[8], d[8];
-  unpack8(*reinterpret_cast<const uint4*>(gamma + o * 8), gm);
+  float bt[8], a[8], mn[8];
   unpack8(*reinterpret_cast<const uint4*>(beta + o * 8), bt);
-  int cur_b = -1;
-  auto coeffs = [&](int b) {
-    const float* st = stats + (long long)b * 2 * groups;
+  long long img_end = 0;  // the walk only moves forward: coefficients are rebuilt when it passes the end of the current image
+  auto coeffs = [&](long long idx) {
+    if (idx < img_end) return;
+    const long long b = idx / per_image;
+    img_end = (b + 1) * per_image;
+    const float* st = stats + b * 2 * groups;
+    float gm[8];  // re-read per image (L1 / L2 hits) rather than held in registers through the walk
+    unpack8(*reinterpret_cast<const uint4*>(gamma + o * 8), gm);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int g = (o * 8 + j) / cpg;
-      const float mean = st[2 * g] * inv_n;
-      const float var = fmaxf(st[2 * g + 1] * inv_n - mean * mean, 0.0f);
-      a[j] = rsqrtf(var + eps) * gm[j];
-      d[j] = fmaf(-mean, a[j], bt[j]);
+      mn[j] = st[2 * g];
+      a[j] = rsqrtf(st[2 * g + 1] + eps) * gm[j];
     }
-    cur_b = b;
   };
   auto one = [&](long long idx, const uint4& v) {
     float f[8];
     unpack8(v, f);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-      float r = fmaf(f[j], a[j], d[j]);
+      float r = fmaf(f[j] - mn[j], a[j], bt[j]);
       if (kSilu) r = __fdividef(r, 1.0f + __expf(-r));  // one ex2 + one rcp on the MUFU unit (a full-precision divide costs ~10 more)
       f[j] = r;
     }
@@ -168,24 +197,21 @@ __global__ void __launch_bounds__(256, 3) groupnorm_apply_kernel(const __nv_bflo
     for (int u = 0; u < 4; ++u) v[u] = *reinterpret_cast<const uint4*>(x + (i + u * stride) * 8);
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-      const int bu = (int)((i + u * stride) / per_image);
-      if (bu != cur_b) coeffs(bu);
+      coeffs(i + u * stride);
       one(i + u * stride, v[u]);
     }
   }
   for (; i + stride < total_octets; i += 2 * stride) {
     const uint4 v0 = *reinterpret_cast<const uint4*>(x + i * 8);
     const uint4 v1 = *reinterpret_cast<const uint4*>(x + (i + stride) * 8);
-    const int b0 = (int)(i / per_image), b1 = (int)((i + stride) / per_image);
-    if (b0 != cur_b) coeffs(b0);
+    coeffs(i);
     one(i, v0);
-    if (b1 != cur_b) coeffs(b1);
+    coeffs(i + stride);
     one(i + stride, v1);
   }
   if (i < total_octets) {
     const uint4 v0 = *reinterpret_cast<const uint4*>(x + i * 8);
-    const int b0 = (int)(i / per_image);
-    if (b0 != cur_b) coeffs(b0);
+    coeffs(i);
     one(i, v0);
   }
 }
@@ -255,8 +281,8 @@ __global__ void __launch_bounds__(256) im2col_scalar_kernel(const T* __restrict_
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Row softmax in place: one block per row, the row is read once into registers (cols <= 8 * 8 * 256 per pass, looped otherwise
-// through a second read: rows of the VAE attention are 1024-65536 long).
+// Row softmax in place: one block per row, three passes over the row at every length (max, sum of exponentials, normalise and
+// store) read the row from memory three times; rows of the VAE attention are 4096-65536 long.
 // ---------------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float block_reduce(float v, float* red, bool is_max) {
   for (int off = 16; off > 0; off >>= 1) {
@@ -363,7 +389,7 @@ extern "C" int ug_groupnorm_bf16(const void* x, void* y, const void* gamma, cons
   float* partial = stats + (long long)batch * groups * 2;
   groupnorm_partial_kernel<<<dim3(chunks, batch), 256, 0, s>>>((const __nv_bfloat16*)x, partial, pixels, c, groups);
   UG_CHECK_LAUNCH("groupnorm_partial");
-  groupnorm_finalize_kernel<<<batch * groups, 32, 0, s>>>(partial, stats, chunks, groups);
+  groupnorm_finalize_kernel<<<batch * groups, 32, 0, s>>>((const __nv_bfloat16*)x, partial, stats, chunks, pixels, c, groups);
   UG_CHECK_LAUNCH("groupnorm_finalize");
   const long long total = (long long)batch * pixels * (c / 8);
   // grid stride (blocks x 256 threads) must be a multiple of c / 8: a thread then keeps one channel octet for its whole walk
